@@ -223,6 +223,17 @@ int lpf_gather_links(const int64_t* links, int64_t bs, const int32_t* idx /* NUL
                      float* xsum, int64_t ld_sum, float* xprod, int64_t ld_prod, const int64_t* n_dev,
                      int x_bf16 /* X holds bf16 (ldx in elements) */, void* stream);
 
+/* Query groups -> links (train/testing.py:14-27: source.repeat(K) x negative targets).  The grouped form holds one
+ * source per query and K targets per query; its flat link index i = q*K + j is link (source[q], targets[q*K + j]).
+ * Writes the flat range of n links that starts at position j0 (0 <= j0 < K) of its first query:
+ *   links[i] = source[(j0 + i) / K],  links[ld + i] = targets[i]   for i < n,
+ * so `source` points at the first query the range touches and `targets` at the range's first target.  Both arrays hold
+ * int32 (id_bytes 4) or int64 (id_bytes 8) ids; links is int64 [2, ld] with ld >= n.  An id outside [0, num_nodes) is
+ * written as 0 (no later kernel reads out of bounds) and sets *bad (int64) to non-zero; the caller resets *bad.
+ * n == 0 is a no-op. */
+int lpf_expand_query_links(const void* source, const void* targets, int32_t id_bytes, int64_t K, int64_t j0, int64_t n,
+                           int64_t num_nodes, int64_t* links, int64_t ld, int64_t* bad, void* stream);
+
 /* dst[r,:] = fill_row[:] for all `rows` rows (skipped when fill_row is NULL), then dst[idx[j],:] = src[j,:]
  * for j < n: puts the pairwise rows of the compacted non-empty links back in batch order, every other link
  * getting the constant empty-set row. */

@@ -205,6 +205,29 @@ __global__ void __launch_bounds__(256) gather_links_kernel(const int64_t* __rest
     }
 }
 
+// ---------------------------------------------------------------------------------------
+// Query groups -> link pairs: links[0, i] = source[(j0 + i) / K], links[1, i] = targets[i] for the flat range
+// i < n of the grouped form (flat index q K + j, the order of the reference's source.repeat(K) x targets).  An id
+// outside [0, num_nodes) is written as 0, so no later kernel reads out of bounds, and raises *bad.
+// ---------------------------------------------------------------------------------------
+template <typename T>
+__global__ void __launch_bounds__(256) expand_query_links_kernel(const T* __restrict__ source,
+                                                                 const T* __restrict__ targets, int64_t K, int64_t j0,
+                                                                 int64_t n, int64_t num_nodes,
+                                                                 int64_t* __restrict__ links, int64_t ld,
+                                                                 int64_t* __restrict__ bad) {
+    bool flag = false;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t t = (int64_t)__ldg(targets + i);
+        const int64_t s = (int64_t)__ldg(source + (j0 + i) / K);     // (consecutive threads: the same cached word)
+        const bool s_ok = s >= 0 && s < num_nodes, t_ok = t >= 0 && t < num_nodes;
+        links[i] = s_ok ? s : 0;
+        links[ld + i] = t_ok ? t : 0;
+        flag |= !(s_ok && t_ok);
+    }
+    if (__any_sync(0xffffffffu, flag) && (threadIdx.x & 31) == 0) *bad = 1;
+}
+
 // dst[r,:] = fill[:] for every row / dst[idx[j],:] = src[j,:]
 __global__ void __launch_bounds__(256) fill_rows_kernel(float* __restrict__ dst, int64_t ldd, int64_t rows, int d,
                                                         const float* __restrict__ fill) {
@@ -303,6 +326,29 @@ extern "C" int lpf_gather_links(const int64_t* links, int64_t bs, const int32_t*
     gather_links_kernel<<<warp_grid(n, 256), 256, 0, (cudaStream_t)stream>>>(links, bs, idx, n, X, ldx, d, xsum, ld_sum,
                                                                              xprod, ld_prod, n_dev, x_bf16);
     return check_launch("lpf_gather_links");
+}
+
+extern "C" int lpf_expand_query_links(const void* source, const void* targets, int32_t id_bytes, int64_t K, int64_t j0,
+                                      int64_t n, int64_t num_nodes, int64_t* links, int64_t ld, int64_t* bad,
+                                      void* stream) {
+    LPF_REQUIRE(id_bytes == 4 || id_bytes == 8, "id_bytes must be 4 or 8");
+    LPF_REQUIRE(K >= 1, "K must be >= 1");
+    LPF_REQUIRE(n >= 0 && j0 >= 0 && j0 < K, "bad range (need n >= 0, 0 <= j0 < K)");
+    LPF_REQUIRE(num_nodes >= 0, "num_nodes < 0");
+    if (n == 0) return LPF_OK;
+    LPF_REQUIRE(source && targets && links && bad, "NULL argument");
+    LPF_REQUIRE(ld >= n, "ld < n");
+    int64_t blocks = (n + 255) / 256;
+    const int64_t cap = (int64_t)kNumSMs * 8;
+    if (blocks > cap) blocks = cap;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (id_bytes == 4)
+        expand_query_links_kernel<int32_t><<<(unsigned)blocks, 256, 0, st>>>(
+            (const int32_t*)source, (const int32_t*)targets, K, j0, n, num_nodes, links, ld, bad);
+    else
+        expand_query_links_kernel<int64_t><<<(unsigned)blocks, 256, 0, st>>>(
+            (const int64_t*)source, (const int64_t*)targets, K, j0, n, num_nodes, links, ld, bad);
+    return check_launch("lpf_expand_query_links");
 }
 
 extern "C" int lpf_scatter_rows(const float* src, int64_t ld_src, const int32_t* idx, int64_t n, float* dst,

@@ -105,12 +105,25 @@ def shard_bounds(num_queries, world, cost=None):
     return bounds
 
 
+def _row_bytes(model, test_set):
+    """float64 [N]: the bytes of a node's adjacency and PPR rows the selection reads (4 deg + 8 nP)."""
+    adj, ppr = model.get_adj(test_set, mask=True), model.get_ppr(test_set)
+    return (4 * (adj.rowptr[1:] - adj.rowptr[:-1]) + 8 * (ppr.rowptr[1:] - ppr.rowptr[:-1])).to(torch.float64)
+
+
+def query_group_cost(model, source, targets, test_set=False):
+    """link_group_cost of the expanded links of query groups (source [Q], targets [Q, K]), from the grouped form: the
+    source's row once, every target's row, 48 bytes per link."""
+    row = _row_bytes(model, test_set)
+    dev = row.device
+    return row[source.to(dev).long()] + row[targets.to(dev).long()].sum(1) + 48.0 * targets.shape[1]
+
+
 def link_group_cost(model, links, group_size, test_set=False):
     """Cost of every group of `group_size` consecutive links: 4 deg + 8 nP (+ 48) bytes of both endpoints' rows, the
     shared source of a citation2-style group counted once (the algorithmic bytes of the selection, SURVEY 8(d))."""
-    adj, ppr = model.get_adj(test_set, mask=True), model.get_ppr(test_set)
-    dev = adj.rowptr.device
-    row = (4 * (adj.rowptr[1:] - adj.rowptr[:-1]) + 8 * (ppr.rowptr[1:] - ppr.rowptr[:-1])).to(torch.float64)
+    row = _row_bytes(model, test_set)
+    dev = row.device
     lk = links.to(dev)
     ng = lk.shape[1] // group_size
     a = lk[0, :ng * group_size].reshape(ng, group_size)
@@ -151,6 +164,132 @@ def score_links_sharded(model, score_func, links, X, test_set=False, group=None,
     return torch.cat(pieces)
 
 
+@torch.no_grad()
+def score_queries_sharded(model, score_func, source, targets, X, test_set=False, group=None, batch_size=None,
+                          balance=True):
+    """score_links_sharded for query groups (source [Q], targets [Q, K], int32 or int64 alike): the queries are sharded
+    over the ranks of `group`, every rank ships and scores only its own (model.score_queries, batch_size links per call
+    rounded down to whole queries), and one all_gather of fp32 scores returns the full [Q, K] on every rank.
+    balance: cut the shards by the weight of the links' rows (shard_bounds / query_group_cost) instead of by count."""
+    world = dist.get_world_size(group) if dist.is_initialized() else 1
+    rank = dist.get_rank(group) if dist.is_initialized() else 0
+    dev = model._dev()
+    source, targets = ops.query_groups(source, targets)
+    Q, K = targets.shape
+    cost = query_group_cost(model, source, targets, test_set) if (balance and world > 1 and hasattr(model, "get_adj")) else None
+    bounds = shard_bounds(Q, world, cost)
+    lo, hi = bounds[rank], bounds[rank + 1]
+    src, tgt = source[lo:hi].to(dev), targets[lo:hi].to(dev)
+    qb = max(1, (batch_size or max(1, (hi - lo) * K)) // max(1, K))
+    outs = [model.score_queries(src[s:s + qb], tgt[s:s + qb], X, score_func, test_set=test_set) for s in range(0, hi - lo, qb)]
+    local = torch.cat(outs) if outs else torch.empty((0, K), device=dev)
+    if world == 1:
+        return local
+    per = max(1, max(bounds[r + 1] - bounds[r] for r in range(world)) * K)
+    pad = torch.zeros(per, dtype=torch.float32, device=dev)
+    pad[:local.numel()] = local.reshape(-1)
+    full = torch.empty(per * world, dtype=torch.float32, device=dev)
+    dist.all_gather_into_tensor(full, pad, group=group)
+    pieces = [full[r * per:r * per + (bounds[r + 1] - bounds[r]) * K] for r in range(world)]
+    return torch.cat(pieces).view(Q, K)
+
+
+class _LinkPairs:
+    """Input of LinkScoreStream.score: int64 link pairs [2, L], staged as they are."""
+
+    def __init__(self, stream, links):
+        self.s, self.lk, self.L, self.on_host = stream, links, links.shape[1], not links.is_cuda
+
+    def stage(self, G):
+        s = self.s
+        if s._stage is None or s._stage[0].shape[1] != G * s.bs:
+            s._stage = [torch.empty((2, G * s.bs), dtype=torch.int64, device=s.dev) for _ in range(2)]
+        return s._stage
+
+    def h2d(self, slot, j, k):
+        # row by row: a strided two-row host slice would go through a slow pitched copy (15 vs 48 GB/s measured)
+        bs, lo = self.s.bs, k * self.s.bs
+        slot[0, j * bs:(j + 1) * bs].copy_(self.lk[0, lo:lo + bs], non_blocking=True)
+        slot[1, j * bs:(j + 1) * bs].copy_(self.lk[1, lo:lo + bs], non_blocking=True)
+
+    def submit(self, P, slot, j, k):
+        bs = self.s.bs
+        P.submit(slot[:, j * bs:(j + 1) * bs] if slot is not None else self.lk[:, k * bs:(k + 1) * bs])
+
+    def links(self, lo, hi):
+        return self.lk[:, lo:hi]
+
+    def begin(self):
+        pass
+
+    def check(self, plan_bad, expanded):
+        pass
+
+
+class _QueryGroups:
+    """Input of LinkScoreStream.score_grouped: source [Q] and targets [Q, K] (int32 or int64), flat link i = q K + j.  A
+    batch is staged as its targets plus the sources it touches and expanded into the plan's links buffer on the device.
+    Out-of-range ids are flagged in word 5 of the plan's header (no selection launch writes it; collect() reads the
+    header back every batch anyway) or, for batches expanded outside a plan, in the stream's own word."""
+
+    def __init__(self, stream, source, targets):
+        self.s, self.src, self.K = stream, source, targets.shape[1]
+        self.tgt = targets.reshape(-1)
+        self.L, self.on_host = self.tgt.numel(), not targets.is_cuda
+        self.S = stream.bs // self.K + 2          # sources a batch of bs links touches at most
+
+    def stage(self, G):
+        s, dt = self.s, self.tgt.dtype          # (kept per id width: callers may alternate int32 and int64 groups)
+        st = s._gstage.get(dt)
+        if st is None or st[0][0].numel() != G * s.bs or st[0][1].numel() != G * self.S:
+            st = s._gstage[dt] = [(torch.empty(G * s.bs, dtype=dt, device=s.dev),
+                                   torch.empty(G * self.S, dtype=dt, device=s.dev)) for _ in range(2)]
+        return st
+
+    def _span(self, lo, hi):
+        return lo // self.K, (hi - 1) // self.K + 1
+
+    def h2d(self, slot, j, k):
+        bs, S, lo = self.s.bs, self.S, k * self.s.bs
+        q0, q1 = self._span(lo, lo + bs)
+        slot[0][j * bs:(j + 1) * bs].copy_(self.tgt[lo:lo + bs], non_blocking=True)
+        slot[1][j * S:j * S + q1 - q0].copy_(self.src[q0:q1], non_blocking=True)
+
+    def submit(self, P, slot, j, k):
+        bs, lo = self.s.bs, k * self.s.bs
+        if slot is not None:
+            src, tgt = slot[1][j * self.S:], slot[0][j * bs:]
+        else:
+            src, tgt = self.src[lo // self.K:], self.tgt[lo:]
+        ops.expand_query_links(src, tgt, self.K, lo % self.K, bs, self.s.num_nodes, P.links, P.hdr[5:6])
+        P.submit(None)
+
+    def links(self, lo, hi):
+        """The int64 links [2, hi - lo] of a flat range, expanded on the device (ragged tail, overflow redo)."""
+        q0, q1 = self._span(lo, hi)
+        dev = self.s.dev
+        out = torch.empty((2, hi - lo), dtype=torch.int64, device=dev)
+        if hi > lo:
+            ops.expand_query_links(self.src[q0:q1].to(dev), self.tgt[lo:hi].to(dev), self.K, lo - q0 * self.K, hi - lo,
+                                   self.s.num_nodes, out, self.s._bad)
+        return out
+
+    def begin(self):
+        """Resets the flags once per call (on the caller's stream, which every plan stream then waits for)."""
+        s = self.s
+        if s._bad is None:
+            s._bad = torch.zeros(1, dtype=torch.int64, device=s.dev)
+        s._bad.zero_()
+        for P in s.plans or []:
+            P.hdr[5:6].zero_()
+
+    def check(self, plan_bad, expanded):
+        """Raises once the call is drained if a plan or an expansion outside the plans met an out-of-range id (the
+        stream's word is read only when such an expansion ran, i.e. after a host round trip the call makes anyway)."""
+        if plan_bad or (expanded and int(self.s._bad.item())):
+            raise _lib.LpfError(f"query groups hold a node id outside [0, {self.s.num_nodes})")
+
+
 class LinkScoreStream:
     """The batch loop of the reference's eval drivers (train/testing.py:25-32, 36-43, 107-117: for every batch
     `elementwise_lin` -> `calc_pairwise` -> `score_func` -> `.cpu()`), pipelined.
@@ -182,11 +321,14 @@ class LinkScoreStream:
         # the non-empty links) overlaps the bandwidth-bound head of the next
         self.streams = [torch.cuda.Stream(device=self.dev) for _ in (self.plans or [])]
         self._stage = None
+        self._gstage = {}
+        self._bad = None
+        self.num_nodes = model._id_bound(self.X, test_set)
         self.batches = 0
 
-    def _sequential(self, links, out_dev):
-        for s in range(0, links.shape[1], max(1, self.bs)):
-            b = links[:, s:s + self.bs]
+    def _sequential(self, inp, out_dev):
+        for s in range(0, inp.L, max(1, self.bs)):
+            b = inp.links(s, min(inp.L, s + self.bs))
             out_dev[s:s + b.shape[1]] = self.model.score_links(b, self.X, self.score_func, test_set=self.test_set,
                                                                return_logits=self.logits)
 
@@ -197,21 +339,45 @@ class LinkScoreStream:
         produced (the reference's per-batch `.cpu()`), complete when the call returns.  Host-resident links and the
         scores travel in groups of `group` batches on a copy stream: the links of group g+1 are on their way while
         group g is scored."""
-        L = links.shape[1]
+        return self._score(_LinkPairs(self, links), out_host, group)
+
+    @torch.no_grad()
+    def score_grouped(self, source, targets, out_host=None, group=4):
+        """score() for query groups: source [Q] and targets [Q, K] (both int32 or both int64; device tensors or pinned
+        host memory) stand for the Q*K links (source[q], targets[q, j]) in that flat order (the reference's citation2
+        eval input, train/testing.py:14-27).  Returns the [Q, K] scores on the device; out_host: a pinned fp32 [Q*K]
+        tensor, as in score().
+
+        The batches are those score() forms on the expanded links — contiguous ranges of batch_size links, which may
+        straddle queries — run in the same order through the same plans.  Host-resident groups ship 4 or 8 bytes per
+        link (the target) plus the few sources a batch touches, instead of 16 bytes per link; each batch is expanded
+        into its plan's links buffer on the device (lpf_expand_query_links).  A node id outside [0, num_nodes) raises
+        LpfError once the call has drained its streams; the stream stays usable."""
+        source, targets = ops.query_groups(source, targets)
+        Q, K = targets.shape
+        if Q * K == 0:
+            return torch.empty((Q, K), dtype=torch.float32, device=self.dev)
+        return self._score(_QueryGroups(self, source, targets), out_host, group).view(Q, K)
+
+    def _score(self, inp, out_host, group):
+        """The pipelined batch loop over the links of `inp` (_LinkPairs or _QueryGroups: how a batch is staged and how
+        it fills a plan's links buffer)."""
+        L = inp.L
         out_dev = torch.empty(L, dtype=torch.float32, device=self.dev)
         main = torch.cuda.current_stream(self.dev)
+        inp.begin()
         if self.plans is None:
-            self._sequential(links, out_dev)
+            self._sequential(inp, out_dev)
             if out_host is not None:
                 out_host.copy_(out_dev)
+            inp.check(False, True)
             return out_dev
         bs, depth = self.bs, len(self.plans)
         nb = L // bs
-        on_host = not links.is_cuda
+        on_host = inp.on_host
         G = max(int(group), depth)
         cs = self.copy_stream
-        if on_host and (self._stage is None or self._stage[0].shape[1] != G * bs):
-            self._stage = [torch.empty((2, G * bs), dtype=torch.int64, device=self.dev) for _ in range(2)]
+        stage = inp.stage(G) if on_host else None
         ev_in = [[torch.cuda.Event() for _ in range(G)] for _ in range(2)]     # [slot][batch of the group]: its links are in
         ev_free = [torch.cuda.Event(), torch.cuda.Event()]
 
@@ -219,13 +385,10 @@ class LinkScoreStream:
             slot = (g // G) % 2
             with torch.cuda.stream(cs):
                 # (the copy stream has already waited for the plans to take the slot's previous links: ev_free)
-                # batch by batch, each announced on its own: the first batch of a call starts after 16 bytes per link of
-                # ITS links have arrived, not after the whole group's; row by row: a strided two-row host slice would go
-                # through a slow pitched copy (15 vs 48 GB/s measured)
+                # batch by batch, each announced on its own: the first batch of a call starts after ITS links have
+                # arrived, not after the whole group's
                 for j in range(min(G, nb - g)):
-                    lo = (g + j) * bs
-                    self._stage[slot][0, j * bs:(j + 1) * bs].copy_(links[0, lo:lo + bs], non_blocking=True)
-                    self._stage[slot][1, j * bs:(j + 1) * bs].copy_(links[1, lo:lo + bs], non_blocking=True)
+                    inp.h2d(stage[slot], j, g + j)
                     ev_in[slot][j].record(cs)
 
         pending = [None] * depth
@@ -239,12 +402,8 @@ class LinkScoreStream:
         for g in range(0, nb, G):
             kb = min(G, nb - g)
             slot = (g // G) % 2
-            if on_host:
-                if g + G < nb:
-                    h2d(g + G)
-                src = self._stage[slot]
-            else:
-                src = links[:, g * bs:(g + kb) * bs]
+            if on_host and g + G < nb:
+                h2d(g + G)
             for j in range(kb):
                 k = g + j
                 P, st = self.plans[k % depth], self.streams[k % depth]
@@ -253,7 +412,7 @@ class LinkScoreStream:
                 with torch.cuda.stream(st):
                     if on_host:
                         st.wait_event(ev_in[slot][j])
-                    P.submit(src[:, j * bs:(j + 1) * bs])
+                    inp.submit(P, stage[slot] if on_host else None, j, k)
                     out_dev[k * bs:(k + 1) * bs].copy_(P.prob, non_blocking=True)
                 pending[k % depth] = k
                 self.batches += 1
@@ -276,6 +435,7 @@ class LinkScoreStream:
         for j, k in enumerate(pending):
             if k is not None and self.plans[j].collect():
                 redo.append(k)
+        plan_bad = any(self.plans[j].last[5] for j, k in enumerate(pending) if k is not None)
         if nb * bs < L:
             redo.append(nb)        # the ragged tail goes through score_links
         for st in self.streams:
@@ -287,7 +447,7 @@ class LinkScoreStream:
             self.model.use_plans = False      # host-sized two-pass path: no pools to overflow
             try:
                 for k in redo:
-                    lk = links[:, k * bs:(k + 1) * bs]
+                    lk = inp.links(k * bs, min(L, (k + 1) * bs))
                     pr = self.model.score_links(lk.to(self.dev), self.X, self.score_func, test_set=self.test_set,
                                                 return_logits=self.logits)
                     out_dev[k * bs:k * bs + pr.numel()] = pr
@@ -297,13 +457,14 @@ class LinkScoreStream:
                 self.model.use_plans = use
             full = [k for k in redo if k < nb]
             if full:                          # larger pools for the batches to come: grown until a batch that overflowed fits
-                probe = links[:, full[0] * bs:(full[0] + 1) * bs].to(self.dev)
+                probe = inp.links(full[0] * bs, (full[0] + 1) * bs).to(self.dev)
                 while True:
                     for P in self.plans:
                         P.grow()
                     if self.plans[0].cap >= 64 * bs or not self.plans[0].run(probe)[1]:
                         break
             main.synchronize()
+        inp.check(plan_bad, bool(redo))
         return out_dev
 
 
@@ -409,17 +570,16 @@ def test_edge_citation2(model, score_func, input_data, h, batch_size, mrr_mode=F
                         stream=None):
     """reference train/testing.py:14-47 with the batch loop pipelined (LinkScoreStream) and the predictions kept
     on the device.  input_data [P, 2] positive edges; mrr_mode: negative_data [P, K] negative targets of each
-    positive's source, result [P, K]; else result [P]."""
+    positive's source, result [P, K]; else result [P].  The negatives are scored as query groups (score_grouped:
+    each positive's source with its K targets), never as a [2, P*K] pair tensor."""
     dev = h.device
-    if mrr_mode:
-        k = negative_data.shape[1]
-        source = input_data.t()[0].reshape(-1, 1).repeat(1, k).reshape(-1)
-        links = torch.stack((source.to(dev), negative_data.reshape(-1).to(dev)))
-    else:
-        links = input_data.t().to(dev).contiguous()
     st = stream if stream is not None else LinkScoreStream(model, score_func, h, batch_size, test_set=test)
-    pred = st.score(links)
-    return pred.view(-1, negative_data.shape[1]) if mrr_mode else pred
+    if mrr_mode:
+        targets = negative_data.to(dev)
+        if targets.dtype not in (torch.int32, torch.int64):
+            targets = targets.long()
+        return st.score_grouped(input_data[:, 0].to(dev, targets.dtype), targets)
+    return st.score(input_data.t().to(dev).contiguous())
 
 
 @torch.no_grad()

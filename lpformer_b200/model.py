@@ -724,6 +724,33 @@ class LinkTransformer(nn.Module):
             ops.link_heads(batch, X_node, consts, prob, idx=sel.nz, zb=zb, logits=return_logits)
         return prob
 
+    @torch.no_grad()
+    def score_queries(self, source, targets, X_node, score_func, test_set=False, return_logits=False):
+        """score_links for query groups: source [Q] and targets [Q, K] (both int32 or both int64, on the device or in
+        pinned host memory) stand for the Q*K links (source[q], targets[q, j]) — the reference's citation2 eval input
+        (train/testing.py:14-27: source.repeat(K) x negative targets).  Returns the [Q, K] scores.
+
+        The groups are expanded into int64 links on the device (lpf_expand_query_links), so only 4 or 8 bytes per link
+        and per query cross the host link instead of 16 per link.  A node id outside [0, num_nodes) raises LpfError."""
+        source, targets = ops.query_groups(source, targets)
+        X_node = self._check_x(X_node)
+        dev = self._dev()
+        Q, K = targets.shape
+        if Q * K == 0:
+            return torch.empty((Q, K), dtype=torch.float32, device=dev)
+        links = torch.empty((2, Q * K), dtype=torch.int64, device=dev)
+        bad = torch.zeros(1, dtype=torch.int64, device=dev)
+        ops.expand_query_links(source.to(dev, non_blocking=True), targets.to(dev, non_blocking=True).reshape(-1), K, 0,
+                               Q * K, self._id_bound(X_node, test_set), links, bad)
+        prob = self.score_links(links, X_node, score_func, test_set=test_set, return_logits=return_logits)
+        if int(bad.item()):                 # (score_links has already waited for the device)
+            raise LpfError(f"query groups hold a node id outside [0, {self._id_bound(X_node, test_set)})")
+        return prob.view(Q, K)
+
+    def _id_bound(self, X_node, test_set):
+        """Node ids index the rows of X_node and of the selection tables."""
+        return min(X_node.shape[0], self.get_adj(test_set, mask=True).n, self.get_ppr(test_set).n)
+
     def _get_plan(self, score_func, consts, X_node, batch, test_set, logits):
         """The sync-free CUDA-graph plan for this batch size (plan.py), or None when the configuration needs the
         host-sized path (generic selection algorithm, i.e. a threshold of 0)."""

@@ -241,6 +241,42 @@ def links_tensor(batch, device) -> torch.Tensor:
     return b.to(device=device, dtype=torch.int64).contiguous()
 
 
+def query_groups(source, targets):
+    """(source [Q], targets [Q, K]) of the grouped form, both int32 or both int64 and on the same device, contiguous.
+    The flat link index q * K + j is link (source[q], targets[q, j]): the order of the reference's source.repeat(K)."""
+    s, t = torch.as_tensor(source), torch.as_tensor(targets)
+    if s.dim() != 1 or t.dim() != 2 or t.shape[0] != s.shape[0]:
+        raise ValueError("query groups must be source [Q] and targets [Q, K] (one source and K targets per query); got "
+                         f"{list(s.shape)} and {list(t.shape)}")
+    if s.dtype != t.dtype or s.dtype not in (torch.int32, torch.int64):
+        raise ValueError(f"source and targets must both be int32 or both int64; got {s.dtype} and {t.dtype}")
+    if s.device != t.device:
+        raise ValueError(f"source and targets must be on the same device; got {s.device} and {t.device}")
+    return s.contiguous(), t.contiguous()
+
+
+def expand_query_links(source, targets, K, j0, n, num_nodes, links, bad):
+    """links[:, :n] = the flat range of n links of the grouped form that starts at position j0 of its first query
+    (lpf_expand_query_links).  source: ids from the first query the range touches on; targets: ids from the range's
+    first target (both 1-D, contiguous, int32 or int64 alike); links: int64 [2, >= n] with unit stride in a row.  Ids
+    outside [0, num_nodes) come out as 0 and set bad (int64 [1]); the caller resets it."""
+    require_cuda(source, targets, links, bad)
+    if source.dtype != targets.dtype or source.dtype not in (torch.int32, torch.int64):
+        raise ValueError(f"source and targets must both be int32 or both int64; got {source.dtype} and {targets.dtype}")
+    if not (source.is_contiguous() and targets.is_contiguous()):
+        raise ValueError("source and targets must be contiguous")
+    if links.dtype != torch.int64 or links.dim() != 2 or links.shape[0] != 2 or links.stride(1) != 1 or links.shape[1] < n:
+        raise ValueError(f"links must be int64 [2, >= {n}] with unit stride in a row")
+    if bad.dtype != torch.int64 or bad.numel() < 1:
+        raise ValueError("bad must be an int64 device word")
+    if n > 0 and K >= 1 and (targets.numel() < n or source.numel() < (j0 + n + K - 1) // K):
+        raise ValueError(f"the range of {n} links at position {j0} needs {(j0 + n + K - 1) // K} sources and {n} targets; "
+                         f"got {source.numel()} and {targets.numel()}")
+    call("lpf_expand_query_links", ptr(source), ptr(targets), source.element_size(), int(K), int(j0), int(n),
+         int(num_nodes), ptr(links), links.stride(0), ptr(bad), stream(), meta=(n,))
+    return links
+
+
 def pick_select_algo(adj: CSR, ppr: CSR, th_1hop, th_non1hop, mode: str) -> int:
     """Intersection-driven kernel when its preconditions hold (thresholds gating PPR-derived sets > 0 and
     all PPR values in (0,1], checked once per table), group width by mean row length; else the generic one."""
