@@ -234,6 +234,37 @@ int lpf_gather_links(const int64_t* links, int64_t bs, const int32_t* idx /* NUL
 int lpf_expand_query_links(const void* source, const void* targets, int32_t id_bytes, int64_t K, int64_t j0, int64_t n,
                            int64_t num_nodes, int64_t* links, int64_t ld, int64_t* bad, void* stream);
 
+/* Source sweep -> links: every node in [0, n_targets) as a target of every source.  Flat link i = q*n_targets + j is
+ * link (source[q], j).  Writes the flat range of n links that starts at position j0 (0 <= j0 < n_targets) of its first
+ * query:  links[i] = source[(j0 + i) / n_targets],  links[ld + i] = (j0 + i) % n_targets   for i < n,
+ * so `source` points at the first query the range touches.  source holds int32 (id_bytes 4) or int64 (id_bytes 8)
+ * ids; n_targets <= num_nodes.  A source outside [0, num_nodes) is written as 0 and sets *bad (int64) to non-zero; the
+ * caller resets *bad.  n == 0 is a no-op. */
+int lpf_expand_source_sweep(const void* source, int32_t id_bytes, int64_t n_targets, int64_t j0, int64_t n,
+                            int64_t num_nodes, int64_t* links, int64_t ld, int64_t* bad, void* stream);
+
+/* Bytes of workspace lpf_topk_fold needs for a range of up to bs scores (-1 for bad arguments). */
+int64_t lpf_topk_fold_workspace_bytes(int64_t bs, int32_t k, int64_t n_targets);
+
+/* Folds the scores prob[0, n) of the flat sweep positions [lo, lo + n) (position q*n_targets + j: source[q], target j)
+ * into per-query state, for num_queries queries:
+ *   top_key fp32 [num_queries, k], top_id int32 [num_queries, k]: the k best candidates so far, ordered by (score
+ *     descending, target id ascending); slots never filled hold (-inf, -1).  Initialise them so before the first fold.
+ *   cnt_ge, cnt_gt int64 [num_queries] (with positives): candidates with score >= / > pos_score[q], accumulated.
+ * The candidates of query q are all j in [0, n_targets) except source[q] and the ids of the exclusion row of source[q]
+ * (ex_rowptr / ex_col: a CSR of ex_rows rows, col ascending within a row; NULL for none; a source outside [0, ex_rows)
+ * has no row).  The counters also leave out positive[q].  source and positive are int32 or int64 (id_bytes), indexed
+ * from query 0; positive, pos_score, cnt_ge and cnt_gt are all given or all NULL.  1 <= k <= 1024.
+ * The state after any sequence of folds depends only on the multiset of (query, target, score) folded, not on how the
+ * positions were cut into ranges or in which order the ranges came.
+ * skip (NULL = never): when *skip is non-zero on the device at launch time, the call folds nothing (a batch whose
+ * scores are invalid, e.g. a pair-pool overflow flag, can be folded later without a host round trip).
+ * workspace: >= lpf_topk_fold_workspace_bytes(n, k, n_targets) bytes.  n == 0 is a no-op. */
+int lpf_topk_fold(const float* prob, int64_t lo, int64_t n, const void* source, const void* positive, int32_t id_bytes,
+                  int64_t num_queries, int64_t n_targets, const int64_t* ex_rowptr, const int32_t* ex_col,
+                  int64_t ex_rows, const float* pos_score, int32_t k, float* top_key, int32_t* top_id, int64_t* cnt_ge,
+                  int64_t* cnt_gt, const int64_t* skip, void* workspace, int64_t workspace_bytes, void* stream);
+
 /* dst[r,:] = fill_row[:] for all `rows` rows (skipped when fill_row is NULL), then dst[idx[j],:] = src[j,:]
  * for j < n: puts the pairwise rows of the compacted non-empty links back in batch order, every other link
  * getting the constant empty-set row. */

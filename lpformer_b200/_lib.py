@@ -46,6 +46,10 @@ SIGNATURES = {
     "lpf_layernorm_act": (_int, [_p, _i64, _p, _p, _p, _i64, _p, _i64, _i64, _i32, _int, _p, _p]),
     "lpf_gather_links": (_int, [_p, _i64, _p, _i64, _p, _i64, _i32, _p, _i64, _p, _i64, _p, _int, _p]),
     "lpf_expand_query_links": (_int, [_p, _p, _i32, _i64, _i64, _i64, _i64, _p, _i64, _p, _p]),
+    "lpf_expand_source_sweep": (_int, [_p, _i32, _i64, _i64, _i64, _i64, _p, _i64, _p, _p]),
+    "lpf_topk_fold_workspace_bytes": (_i64, [_i64, _i32, _i64]),
+    "lpf_topk_fold": (_int, [_p, _i64, _i64, _p, _p, _i32, _i64, _i64, _p, _p, _i64, _p, _i32, _p, _p, _p, _p, _p, _p,
+                             _i64, _p]),
     "lpf_scatter_rows": (_int, [_p, _i64, _p, _i64, _p, _i64, _i64, _i32, _p, _p]),
     "lpf_debug_heads_clocks": (_int, [_p]),
     "lpf_debug_select_clocks": (_int, [_p]),
@@ -117,7 +121,7 @@ def load():
 
 # kernels launched per entry point (for bench.py's gpu_launches and per-kernel CUDA-event timing)
 KERNEL_LAUNCHES = {"lpf_select_count": 3, "lpf_scan_counts": 2, "lpf_select_fill": 2, "lpf_rpe_hidden": 1,
-                   "lpf_gemm": 1, "lpf_gemm_tc": 1, "lpf_pack_weight": 1, "lpf_layernorm_act": 1, "lpf_gather_links": 1, "lpf_expand_query_links": 1, "lpf_attend_fused": 1, "lpf_attend_fused_ws": 2,
+                   "lpf_gemm": 1, "lpf_gemm_tc": 1, "lpf_pack_weight": 1, "lpf_layernorm_act": 1, "lpf_gather_links": 1, "lpf_expand_query_links": 1, "lpf_expand_source_sweep": 1, "lpf_topk_fold": 2, "lpf_attend_fused": 1, "lpf_attend_fused_ws": 2,
                    "lpf_gcn_spmm": 1, "lpf_gcn_layer": 1, "lpf_nz_links_fused": 2, "lpf_nz_pairs": 1, "lpf_select_compact": 2, "lpf_select_onepass": 4, "lpf_select_onepass_packed": 6, "lpf_pack_link_rows": 4, "lpf_scatter_rows": 2, "lpf_link_heads_tc": 1, "lpf_link_heads_f16": 1, "lpf_pack_weight_f16": 1}
 
 

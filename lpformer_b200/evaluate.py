@@ -8,11 +8,19 @@ replicated by ONE all-gather over NCCL/NVLink (SURVEY.md §8e).
 """
 from __future__ import annotations
 
+from collections import namedtuple
+
 import torch
 import torch.distributed as dist
 
 from . import _lib, ops
+from .graph import csr_from_sparse
 from .plan import ScorePlan
+
+TopTargets = namedtuple("TopTargets", "scores targets rank")
+TopTargets.__doc__ = """LinkScoreStream.top_targets / top_targets_sharded: scores fp32 [Q, k] and targets int64 [Q, k] of every
+query's k best candidates (score descending, then target id ascending; (-inf, -1) where a query has fewer than k
+candidates), rank fp32 [Q] of the positives among the filtered candidates (None without positives)."""
 
 
 @torch.no_grad()
@@ -194,7 +202,54 @@ def score_queries_sharded(model, score_func, source, targets, X, test_set=False,
     return torch.cat(pieces).view(Q, K)
 
 
-class _LinkPairs:
+@torch.no_grad()
+def top_targets_sharded(model, score_func, source, X, k, exclude=None, positive=None, test_set=False, group=None,
+                        batch_size=None, stream=None):
+    """LinkScoreStream.top_targets with the queries sharded over the ranks of `group`: every query costs one sweep of
+    all N nodes, so the shards are cut by count (shard_bounds); each rank runs its own stream (`stream`, or one of
+    batch_size links, default 2^21) on its queries, and ONE all_gather of the padded [Q_r, k] results (plus the ranks)
+    returns the full TopTargets on every rank."""
+    world = dist.get_world_size(group) if dist.is_initialized() else 1
+    rank = dist.get_rank(group) if dist.is_initialized() else 0
+    src = torch.as_tensor(source)
+    Q = src.shape[0]
+    bounds = shard_bounds(Q, world)
+    lo, hi = bounds[rank], bounds[rank + 1]
+    st = stream if stream is not None else LinkScoreStream(model, score_func, X, batch_size or (1 << 21),
+                                                           test_set=test_set)
+    mine = st.top_targets(src[lo:hi], k, exclude=exclude,
+                          positive=None if positive is None else torch.as_tensor(positive)[lo:hi])
+    if world == 1:
+        return mine
+    # one float64 row per query: k scores, k target ids and the rank (all exact in float64)
+    per = max(1, max(bounds[r + 1] - bounds[r] for r in range(world)))
+    w = 2 * k + (positive is not None)
+    pad = torch.zeros((per, w), dtype=torch.float64, device=mine.scores.device)
+    pad[:hi - lo, :k] = mine.scores
+    pad[:hi - lo, k:2 * k] = mine.targets.to(torch.float64)
+    if positive is not None:
+        pad[:hi - lo, 2 * k] = mine.rank
+    full = torch.empty((per * world, w), dtype=torch.float64, device=pad.device)
+    dist.all_gather_into_tensor(full, pad, group=group)
+    rows = torch.cat([full[r * per:r * per + bounds[r + 1] - bounds[r]] for r in range(world)])
+    return TopTargets(rows[:, :k].float(), rows[:, k:2 * k].long(), rows[:, 2 * k].float() if positive is not None else None)
+
+
+class _Input:
+    """What the batch loop does with a batch's scores: by default they go into the [L] output at their flat position."""
+    out = None
+
+    def alloc(self):
+        self.out = torch.empty(self.L, dtype=torch.float32, device=self.s.dev)
+        return self.out
+
+    def take(self, prob, lo, P=None):
+        """prob: the scores of flat positions [lo, lo + prob.numel()), on the current stream; P: the plan that produced
+        them (None: scored outside the plans)."""
+        self.out[lo:lo + prob.numel()].copy_(prob, non_blocking=True)
+
+
+class _LinkPairs(_Input):
     """Input of LinkScoreStream.score: int64 link pairs [2, L], staged as they are."""
 
     def __init__(self, stream, links):
@@ -226,11 +281,12 @@ class _LinkPairs:
         pass
 
 
-class _QueryGroups:
+class _QueryGroups(_Input):
     """Input of LinkScoreStream.score_grouped: source [Q] and targets [Q, K] (int32 or int64), flat link i = q K + j.  A
     batch is staged as its targets plus the sources it touches and expanded into the plan's links buffer on the device.
     Out-of-range ids are flagged in word 5 of the plan's header (no selection launch writes it; collect() reads the
     header back every batch anyway) or, for batches expanded outside a plan, in the stream's own word."""
+    what = "query groups hold a node id"
 
     def __init__(self, stream, source, targets):
         self.s, self.src, self.K = stream, source, targets.shape[1]
@@ -287,7 +343,61 @@ class _QueryGroups:
         """Raises once the call is drained if a plan or an expansion outside the plans met an out-of-range id (the
         stream's word is read only when such an expansion ran, i.e. after a host round trip the call makes anyway)."""
         if plan_bad or (expanded and int(self.s._bad.item())):
-            raise _lib.LpfError(f"query groups hold a node id outside [0, {self.s.num_nodes})")
+            raise _lib.LpfError(f"{self.what} outside [0, {self.s.num_nodes})")
+
+
+class _SourceSweep(_QueryGroups):
+    """Input of LinkScoreStream.top_targets: the query groups (source[q], every node j < N), flat link i = q N + j,
+    never materialised.  Each batch is expanded on the device (lpf_expand_source_sweep) and its scores are folded into
+    per-query top-k state and rank counters (lpf_topk_fold) instead of being kept: no [L] output exists."""
+    what = "sources hold a node id"
+
+    def __init__(self, stream, source, k, exclude, positive, pos_score):
+        self.s, self.src, self.K = stream, source, stream.num_nodes
+        self.L, self.on_host = source.numel() * self.K, False
+        Q, dev = source.numel(), stream.dev
+        self.k, self.exclude, self.positive, self.pos_score = k, exclude, positive, pos_score
+        self.top_key = torch.full((Q, k), float("-inf"), dtype=torch.float32, device=dev)
+        self.top_id = torch.full((Q, k), -1, dtype=torch.int32, device=dev)
+        self.cnt = torch.zeros((2, Q), dtype=torch.int64, device=dev) if positive is not None else None
+        self.ws = ops.topk_fold_workspace(stream.bs, k, self.K, dev)
+
+    def submit(self, P, slot, j, k):
+        bs, lo = self.s.bs, k * self.s.bs
+        ops.expand_source_sweep(self.src[lo // self.K:], self.K, lo % self.K, bs, self.s.num_nodes, P.links, P.hdr[5:6])
+        P.submit(None)
+
+    def links(self, lo, hi):
+        """The int64 links [2, hi - lo] of a flat range, expanded on the device (ragged tail, overflow redo)."""
+        q0 = lo // self.K
+        out = torch.empty((2, hi - lo), dtype=torch.int64, device=self.s.dev)
+        if hi > lo:
+            ops.expand_source_sweep(self.src[q0:], self.K, lo - q0 * self.K, hi - lo, self.s.num_nodes, out, self.s._bad)
+        return out
+
+    def alloc(self):
+        return None
+
+    def take(self, prob, lo, P=None):
+        """Folds the scores.  The folds of one call update the same state, so they run one after another on the
+        stream's fold stream: a plan's batch is folded there once its launch is through, with the plan's overflow word
+        as the skip word (an overflowed batch is folded when it is re-scored, in any order: the fold's result does not
+        depend on it), and the plan's next batch waits until the fold has read the plan's scores.  Scores produced
+        outside the plans are folded on the current stream, after every plan stream has drained."""
+        if P is None:
+            self._fold(prob, lo, None)
+            return
+        cur, fs = torch.cuda.current_stream(self.s.dev), self.s.fold_stream
+        fs.wait_stream(cur)
+        with torch.cuda.stream(fs):
+            self._fold(prob, lo, P.hdr[4:5])
+        cur.wait_stream(fs)
+
+    def _fold(self, prob, lo, skip):
+        c = self.cnt
+        ops.topk_fold(prob, lo, self.src, self.K, self.k, self.top_key, self.top_id, self.ws, exclude=self.exclude,
+                      positive=self.positive, pos_score=self.pos_score, cnt_ge=None if c is None else c[0],
+                      cnt_gt=None if c is None else c[1], skip=skip)
 
 
 class LinkScoreStream:
@@ -320,17 +430,18 @@ class LinkScoreStream:
         # every plan launches on a stream of its own: the latency-bound tail of one batch (hub sources, heavy links,
         # the non-empty links) overlaps the bandwidth-bound head of the next
         self.streams = [torch.cuda.Stream(device=self.dev) for _ in (self.plans or [])]
+        self.fold_stream = torch.cuda.Stream(device=self.dev)     # top_targets: the folds, one after another
         self._stage = None
         self._gstage = {}
         self._bad = None
         self.num_nodes = model._id_bound(self.X, test_set)
         self.batches = 0
 
-    def _sequential(self, inp, out_dev):
+    def _sequential(self, inp):
         for s in range(0, inp.L, max(1, self.bs)):
             b = inp.links(s, min(inp.L, s + self.bs))
-            out_dev[s:s + b.shape[1]] = self.model.score_links(b, self.X, self.score_func, test_set=self.test_set,
-                                                               return_logits=self.logits)
+            inp.take(self.model.score_links(b, self.X, self.score_func, test_set=self.test_set,
+                                            return_logits=self.logits), s)
 
     @torch.no_grad()
     def score(self, links, out_host=None, group=4):
@@ -359,15 +470,64 @@ class LinkScoreStream:
             return torch.empty((Q, K), dtype=torch.float32, device=self.dev)
         return self._score(_QueryGroups(self, source, targets), out_host, group).view(Q, K)
 
+    @torch.no_grad()
+    def top_targets(self, source, k, exclude=None, positive=None):
+        """Top-k retrieval over every node: for each source[q] the k targets with the highest scores among all N nodes
+        (N = the stream's node-id bound) except the source itself and, with `exclude`, the source's row of that
+        adjacency (anything graph.csr_from_sparse accepts; a filtered evaluation passes model.get_adj(False,
+        mask=True)).  The scores are this stream's: probabilities, or logits with return_logits.
+
+        positive [Q] (optional): rank of each positive among the same filtered candidates (the positive left out),
+        1 + (#(score >= s_pos) + #(score > s_pos)) / 2 — get_ranking_list's convention with those candidates as the
+        negatives — where s_pos is the positive link's score from score().
+
+        source / positive: int32 or int64, on the device or in host memory.  Returns TopTargets(scores fp32 [Q, k],
+        targets int64 [Q, k], rank fp32 [Q] or None) on the device.  The Q x N candidate links run through the same
+        batches and plans as score() — expanded on the device batch by batch and folded there into a fixed [Q, k]
+        state (lpf_topk_fold) — and are never materialised.  A source or positive outside [0, N), or a positive equal to
+        its source, raises LpfError."""
+        src = torch.as_tensor(source)
+        if src.dim() != 1 or src.dtype not in (torch.int32, torch.int64):
+            raise ValueError(f"source must be a 1-D int32 or int64 tensor; got {src.dtype} {list(src.shape)}")
+        k = int(k)
+        if not 1 <= k <= 1024:
+            raise ValueError(f"k must be in [1, 1024]; got {k}")
+        if self.bs < 1:
+            raise ValueError("top_targets needs a batch size >= 1")
+        src = src.to(self.dev).contiguous()
+        Q, N = src.numel(), self.num_nodes
+        if Q > 0 and bool(((src < 0) | (src >= N)).any()):
+            raise _lib.LpfError(f"sources hold a node id outside [0, {N})")
+        pos = pos_score = None
+        if positive is not None:
+            pos = torch.as_tensor(positive)
+            if pos.shape != src.shape or pos.dtype not in (torch.int32, torch.int64):
+                raise ValueError(f"positive must be int32 or int64 [{Q}]; got {pos.dtype} {list(pos.shape)}")
+            pos = pos.to(self.dev, src.dtype).contiguous()
+            if Q > 0 and bool(((pos < 0) | (pos >= N) | (pos == src)).any()):
+                raise _lib.LpfError(f"positives must be node ids in [0, {N}) other than their source")
+        if Q == 0:
+            return TopTargets(torch.empty((0, k), dtype=torch.float32, device=self.dev),
+                              torch.empty((0, k), dtype=torch.int64, device=self.dev),
+                              None if pos is None else torch.empty(0, dtype=torch.float32, device=self.dev))
+        if pos is not None:
+            pos_score = self.score(torch.stack((src.long(), pos.long())))
+        ex = None if exclude is None else csr_from_sparse(exclude, device=self.dev, mask=True)
+        inp = _SourceSweep(self, src, k, ex, pos, pos_score)
+        self._score(inp, None, 4)
+        rank = None if pos is None else 0.5 * (inp.cnt[0] + inp.cnt[1]).to(torch.float32) + 1
+        return TopTargets(inp.top_key, inp.top_id.long(), rank)
+
     def _score(self, inp, out_host, group):
-        """The pipelined batch loop over the links of `inp` (_LinkPairs or _QueryGroups: how a batch is staged and how
-        it fills a plan's links buffer)."""
+        """The pipelined batch loop over the links of `inp` (_LinkPairs, _QueryGroups or _SourceSweep: how a batch is
+        staged, how it fills a plan's links buffer and what becomes of its scores).  Returns the [L] scores (None for
+        an input that keeps none)."""
         L = inp.L
-        out_dev = torch.empty(L, dtype=torch.float32, device=self.dev)
+        out_dev = inp.alloc()
         main = torch.cuda.current_stream(self.dev)
         inp.begin()
         if self.plans is None:
-            self._sequential(inp, out_dev)
+            self._sequential(inp)
             if out_host is not None:
                 out_host.copy_(out_dev)
             inp.check(False, True)
@@ -413,7 +573,7 @@ class LinkScoreStream:
                     if on_host:
                         st.wait_event(ev_in[slot][j])
                     inp.submit(P, stage[slot] if on_host else None, j, k)
-                    out_dev[k * bs:(k + 1) * bs].copy_(P.prob, non_blocking=True)
+                    inp.take(P.prob, k * bs, P)
                 pending[k % depth] = k
                 self.batches += 1
             if on_host or out_host is not None:
@@ -450,7 +610,7 @@ class LinkScoreStream:
                     lk = inp.links(k * bs, min(L, (k + 1) * bs))
                     pr = self.model.score_links(lk.to(self.dev), self.X, self.score_func, test_set=self.test_set,
                                                 return_logits=self.logits)
-                    out_dev[k * bs:k * bs + pr.numel()] = pr
+                    inp.take(pr, k * bs)
                     if out_host is not None:
                         out_host[k * bs:k * bs + pr.numel()].copy_(pr)
             finally:
@@ -485,12 +645,27 @@ def get_ranking_list(y_pred_pos, y_pred_neg):
 
 
 @torch.no_grad()
-def evaluate_mrr(y_pred_pos, y_pred_neg):
-    """reference train/evaluation.py:23-50: Hits@{10,50,100} and MRR of the ranking list."""
-    rank = get_ranking_list(y_pred_pos, y_pred_neg)
+def ranking_metrics(rank):
+    """reference train/evaluation.py:23-50 from the ranks: Hits@{10,50,100} and MRR."""
     res = torch.stack([(rank <= 10).float().mean(), (rank <= 50).float().mean(), (rank <= 100).float().mean(),
                        (1.0 / rank).mean()]).tolist()
     return {"Hits@10": res[0], "Hits@50": res[1], "Hits@100": res[2], "MRR": res[3]}
+
+
+@torch.no_grad()
+def evaluate_mrr(y_pred_pos, y_pred_neg):
+    """reference train/evaluation.py:23-50: Hits@{10,50,100} and MRR of the ranking list."""
+    return ranking_metrics(get_ranking_list(y_pred_pos, y_pred_neg))
+
+
+@torch.no_grad()
+def evaluate_full_ranking(model, score_func, source, positive, X, exclude=None, test_set=False, group=None,
+                          batch_size=None, stream=None):
+    """Filtered full-ranking Hits@{10,50,100} and MRR: every positive (source[q], positive[q]) ranked among ALL nodes
+    but the source and its row of `exclude` (top_targets_sharded) instead of among sampled negatives."""
+    return ranking_metrics(top_targets_sharded(model, score_func, source, X, 1, exclude=exclude, positive=positive,
+                                               test_set=test_set, group=group, batch_size=batch_size,
+                                               stream=stream).rank)
 
 
 @torch.no_grad()

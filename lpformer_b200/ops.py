@@ -277,6 +277,80 @@ def expand_query_links(source, targets, K, j0, n, num_nodes, links, bad):
     return links
 
 
+def _ids(name, t):
+    if t.dtype not in (torch.int32, torch.int64) or t.dim() != 1 or not t.is_contiguous():
+        raise ValueError(f"{name} must be a contiguous 1-D int32 or int64 tensor; got {t.dtype} {list(t.shape)}")
+
+
+def expand_source_sweep(source, n_targets, j0, n, num_nodes, links, bad):
+    """links[:, :n] = the flat range of n links of the source sweep (link q * n_targets + j is (source[q], j)) that
+    starts at position j0 of its first query (lpf_expand_source_sweep).  source: ids from the first query the range
+    touches on (1-D, contiguous, int32 or int64); links: int64 [2, >= n] with unit stride in a row.  A source outside
+    [0, num_nodes) comes out as 0 and sets bad (int64 [1]); the caller resets it."""
+    _ids("source", source)
+    if links.dtype != torch.int64 or links.dim() != 2 or links.shape[0] != 2 or links.stride(1) != 1 or links.shape[1] < n:
+        raise ValueError(f"links must be int64 [2, >= {n}] with unit stride in a row")
+    if bad.dtype != torch.int64 or bad.numel() < 1:
+        raise ValueError("bad must be an int64 device word")
+    if n > 0 and n_targets >= 1 and source.numel() < (j0 + n + n_targets - 1) // n_targets:
+        raise ValueError(f"the range of {n} links at position {j0} needs {(j0 + n + n_targets - 1) // n_targets} "
+                         f"sources; got {source.numel()}")
+    require_cuda(source, links, bad)
+    call("lpf_expand_source_sweep", ptr(source), source.element_size(), int(n_targets), int(j0), int(n),
+         int(num_nodes), ptr(links), links.stride(0), ptr(bad), stream(), meta=(n,))
+    return links
+
+
+def topk_fold_workspace(bs, k, n_targets, device):
+    """A workspace for lpf_topk_fold over ranges of up to bs scores."""
+    nbytes = _lib.load().lpf_topk_fold_workspace_bytes(int(bs), int(k), int(n_targets))
+    if nbytes < 0:
+        raise ValueError(f"bad top-k workspace arguments (bs {bs}, k {k}, n_targets {n_targets}; 1 <= k <= 1024)")
+    return torch.empty(max(1, nbytes), dtype=torch.uint8, device=device)
+
+
+def topk_fold(prob, lo, source, n_targets, k, top_key, top_id, workspace, exclude=None, positive=None,
+              pos_score=None, cnt_ge=None, cnt_gt=None, skip=None):
+    """Folds prob [n] — the scores of the sweep positions [lo, lo + n) — into the per-query state (lpf_topk_fold):
+    top_key fp32 / top_id int32 [Q, k] (the k best candidates, score descending then id ascending; (-inf, -1) while
+    unfilled) and, with positive [Q] / pos_score fp32 [Q], cnt_ge / cnt_gt int64 [Q] (candidates with score >= / > the
+    positive's).  Candidates: every target in [0, n_targets) but the source and its row of `exclude` (a CSR or None);
+    the counters also leave out the positive.  skip: an int64 device word; non-zero at launch time = fold nothing."""
+    _ids("source", source)
+    Q = source.numel()
+    if prob.dtype != torch.float32 or prob.dim() != 1 or not prob.is_contiguous():
+        raise ValueError("prob must be a contiguous fp32 [n] tensor")
+    if not 1 <= int(k) <= 1024:
+        raise ValueError(f"k must be in [1, 1024]; got {k}")
+    if top_key.dtype != torch.float32 or top_id.dtype != torch.int32 or tuple(top_key.shape) != (Q, k) or \
+            tuple(top_id.shape) != (Q, k) or not (top_key.is_contiguous() and top_id.is_contiguous()):
+        raise ValueError(f"top_key / top_id must be contiguous fp32 / int32 [{Q}, {k}]")
+    given = [t is not None for t in (positive, pos_score, cnt_ge, cnt_gt)]
+    if any(given) and not all(given):
+        raise ValueError("positive, pos_score, cnt_ge and cnt_gt go together")
+    if positive is not None:
+        _ids("positive", positive)
+        if positive.dtype != source.dtype or positive.numel() != Q:
+            raise ValueError(f"positive must be [{Q}] of the source's dtype ({source.dtype})")
+        if pos_score.dtype != torch.float32 or pos_score.numel() != Q or not pos_score.is_contiguous():
+            raise ValueError(f"pos_score must be a contiguous fp32 [{Q}] tensor")
+        for c in (cnt_ge, cnt_gt):
+            if c.dtype != torch.int64 or c.numel() != Q or not c.is_contiguous():
+                raise ValueError(f"cnt_ge / cnt_gt must be contiguous int64 [{Q}] tensors")
+    if skip is not None and (skip.dtype != torch.int64 or skip.numel() < 1):
+        raise ValueError("skip must be an int64 device word")
+    require_cuda(prob, source, top_key, top_id, workspace, positive, pos_score, cnt_ge, cnt_gt, skip)
+    if exclude is not None:
+        require_cuda(exclude.rowptr, exclude.col)
+        if exclude.nnz == 0:          # (no row to look up; an empty col may have no storage)
+            exclude = None
+    n = prob.numel()
+    call("lpf_topk_fold", ptr(prob), int(lo), n, ptr(source), ptr(positive), source.element_size(), Q, int(n_targets),
+         None if exclude is None else ptr(exclude.rowptr), None if exclude is None else ptr(exclude.col),
+         0 if exclude is None else exclude.n, ptr(pos_score), int(k), ptr(top_key), ptr(top_id), ptr(cnt_ge),
+         ptr(cnt_gt), ptr(skip), ptr(workspace), workspace.numel(), stream(), meta=(n,))
+
+
 def pick_select_algo(adj: CSR, ppr: CSR, th_1hop, th_non1hop, mode: str) -> int:
     """Intersection-driven kernel when its preconditions hold (thresholds gating PPR-derived sets > 0 and
     all PPR values in (0,1], checked once per table), group width by mean row length; else the generic one."""
