@@ -487,6 +487,64 @@ void* lpf_ppr_push_host(const int64_t* indptr_host, const int32_t* indices_host,
                         double alpha, double eps, int nthreads, int64_t* nnz);
 int lpf_ppr_push_host_fetch(void* handle, int64_t* rowptr_host, int32_t* col_host, float* val_host);
 
+/* ------------------------------------------------------------------------- *
+ * Backward pass (training at dropout 0): the gradients of the host-sized forward with respect to the reference's
+ * parameters and to X_node.  Parameter gradients are reduced deterministically through a caller-owned workspace
+ * (size from the matching *_workspace_bytes; -1 = bad arguments); `accumulate` != 0 adds into the outputs instead of
+ * overwriting them.  Scatters into node-indexed tables (dX, dKV) are fp32 atomic adds into zero-initialised tables.
+ *
+ * lpf_layernorm_act_backward: y = act(LN(x)) of lpf_layernorm_act (nn.LayerNorm + F.relu of MLP, post_att_norm, the GCN's
+ *   lns / gnn_norm; models/other_models.py:66-72,125-133, modules/layers.py:80) from the saved pre-norm rows x:
+ *   dX (+)= dx, dgamma / dbeta (+)= column sums.  gamma == beta == NULL: ReLU (or identity) only.  n <= 1024.
+ * lpf_gemm_wgrad: dW[N,K] (+)= dY[M,N]^T A[M,K] and db[N] (+)= sum of dY's rows, for nn.Linear / GCNConv.lin /
+ *   lin_l / lin_r / the RPE contraction over M links, pairs or nodes (rows split over the grid, fp32 FFMA).  dW or db
+ *   may be NULL (A may be NULL when dW is).  dX = dY W goes through lpf_gemm_tc on the transposed weight.
+ * lpf_act_backward: dX = dY [Y > 0] (act = LPF_EPI_RELU) or dY Y (1 - Y) (LPF_EPI_SIGMOID) from the saved output Y
+ *   (MLP without norm, mlp_score; models/other_models.py:173-179).
+ * lpf_gather_links_backward: the transpose of lpf_gather_links (X[a] * X[b] of elementwise_lin, X[a] + X[b] into lin_l;
+ *   models/link_transformer.py:100-101, modules/layers.py:208-214): dX[a] += dsum + dprod X[b], dX[b] += dsum + dprod X[a].
+ * lpf_scatter_rows_backward: the transpose of lpf_scatter_rows with a fill row: dsrc[j] = dG[idx[j]] (dsrc may be NULL)
+ *   and dfill = the sum of the rows of dG that idx does not name (the shared pairwise row of the links with empty sets).
+ * lpf_rpe_hidden_backward: the first Linear + LayerNorm + ReLU of a PPR encoder (get_pos_encodings,
+ *   models/link_transformer.py:182-211), both orderings (pa, pb) and (pb, pa), from dh = d hsum of rows
+ *   [row0, row0 + rows) (dh row r belongs to pair row0 + r): dw1 [d, 2], db1, dln_w, dln_b.  d <= 256.
+ * lpf_attend_backward: the segment-softmax attention of lpf_attend_fused_ws (modules/layers.py:39-82, :161-224) for the
+ *   links of the batch (or the positions in idx), one warp per link at any set size, with its row map (r_map / r_const).
+ *   From dY (the gradient of the layer's output rows, first heads*ch columns) it writes dQ [n, heads*ch], dR per pair row
+ *   (rows the map names; every other pair's gradient is added into dR_const [3, heads*ch] by type), adds into dKV [N,
+ *   heads*ch] and writes link_rows [n, 4 heads*ch] = (d o | dY LN-normalised o | dY | d att) per link, whose column
+ *   sums (lpf_gemm_wgrad with dW = NULL) are the gradients of bias, post_att_norm.weight, post_att_norm.bias and att.
+ * ------------------------------------------------------------------------- */
+int64_t lpf_layernorm_act_backward_workspace_bytes(int64_t rows, int32_t n);
+int lpf_layernorm_act_backward(const float* X, int64_t ldx, const float* gamma, const float* beta, int relu,
+                               const float* dY, int64_t lddy, float* dX, int64_t lddx, int accumulate_dx,
+                               float* dgamma, float* dbeta, int accumulate_param, int64_t rows, int32_t n,
+                               void* workspace, int64_t workspace_bytes, void* stream);
+int64_t lpf_gemm_wgrad_workspace_bytes(int64_t M, int32_t N, int32_t K);
+int lpf_gemm_wgrad(const float* A, int64_t lda, const float* dY, int64_t lddy, int64_t M, int32_t N, int32_t K,
+                   float* dW, int64_t ldw, float* db, int accumulate, void* workspace, int64_t workspace_bytes,
+                   void* stream);
+int lpf_act_backward(const float* Y, int64_t ldy, const float* dY, int64_t lddy, float* dX, int64_t lddx,
+                     int64_t rows, int32_t n, int act, void* stream);
+int lpf_gather_links_backward(const int64_t* links, int64_t bs, const int32_t* idx, int64_t n, const float* X,
+                              int64_t ldx, int32_t d, const float* dsum, int64_t ld_sum, const float* dprod,
+                              int64_t ld_prod, float* dX, int64_t lddx, void* stream);
+int64_t lpf_scatter_rows_backward_workspace_bytes(int64_t rows, int32_t d);
+int lpf_scatter_rows_backward(const float* dG, int64_t ldg, int64_t rows, int32_t d, const int32_t* idx, int64_t n,
+                              float* dsrc, int64_t ld_src, float* dfill, void* workspace, int64_t workspace_bytes,
+                              void* stream);
+int64_t lpf_rpe_hidden_backward_workspace_bytes(int64_t rows, int32_t d);
+int lpf_rpe_hidden_backward(const float* src_ppr, const float* tgt_ppr, int64_t row0, int64_t rows,
+                            const float* w1, const float* b1, const float* ln_w, const float* ln_b, int32_t d,
+                            const float* dh, int64_t ld_dh, float* dw1, float* db1, float* dln_w, float* dln_b,
+                            int accumulate, void* workspace, int64_t workspace_bytes, void* stream);
+int lpf_attend_backward(const int64_t* ptr, int64_t bs, const int32_t* idx, int64_t n, const int32_t* node,
+                        const float* KV, int64_t ld_kv, const float* R, int64_t ld_r, const int32_t* r_map,
+                        const float* r_const, const float* Q, int64_t ld_q, const float* att, const float* bias,
+                        const float* ln_w, const float* ln_b, int32_t heads, int32_t ch, const float* dY,
+                        int64_t ld_dy, float* dR, int64_t ld_dr, float* dR_const, float* dQ, int64_t ld_dq,
+                        float* dKV, int64_t ld_dkv, float* link_rows, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

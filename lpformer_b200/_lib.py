@@ -77,6 +77,21 @@ SIGNATURES = {
     "lpf_ppr_push_host_fetch": (_int, [_p, _p, _p, _p]),
     "lpf_gcn_spmm": (_int, [_p, _p, _p, _i64, _i64, _p, _i64, _p, _i32, _p, _i64, _p]),
     "lpf_gcn_layer": (_int, [_p, _p, _p, _i64, _i64, _p, _i64, _p, _i32, _p, _p, _int, _p, _i64, _p, _p, _p, _i64, _p]),
+    # backward pass (csrc/backward.cu)
+    "lpf_layernorm_act_backward_workspace_bytes": (_i64, [_i64, _i32]),
+    "lpf_layernorm_act_backward": (_int, [_p, _i64, _p, _p, _int, _p, _i64, _p, _i64, _int, _p, _p, _int, _i64, _i32, _p,
+                                          _i64, _p]),
+    "lpf_gemm_wgrad_workspace_bytes": (_i64, [_i64, _i32, _i32]),
+    "lpf_gemm_wgrad": (_int, [_p, _i64, _p, _i64, _i64, _i32, _i32, _p, _i64, _p, _int, _p, _i64, _p]),
+    "lpf_act_backward": (_int, [_p, _i64, _p, _i64, _p, _i64, _i64, _i32, _int, _p]),
+    "lpf_gather_links_backward": (_int, [_p, _i64, _p, _i64, _p, _i64, _i32, _p, _i64, _p, _i64, _p, _i64, _p]),
+    "lpf_scatter_rows_backward_workspace_bytes": (_i64, [_i64, _i32]),
+    "lpf_scatter_rows_backward": (_int, [_p, _i64, _i64, _i32, _p, _i64, _p, _i64, _p, _p, _i64, _p]),
+    "lpf_rpe_hidden_backward_workspace_bytes": (_i64, [_i64, _i32]),
+    "lpf_rpe_hidden_backward": (_int, [_p, _p, _i64, _i64, _p, _p, _p, _p, _i32, _p, _i64, _p, _p, _p, _p, _int, _p, _i64,
+                                       _p]),
+    "lpf_attend_backward": (_int, [_p, _i64, _p, _i64, _p, _p, _i64, _p, _i64, _p, _p, _p, _i64, _p, _p, _p, _p, _i32,
+                                   _i32, _p, _i64, _p, _i64, _p, _p, _i64, _p, _i64, _p, _p]),
 }
 
 
@@ -122,7 +137,9 @@ def load():
 # kernels launched per entry point (for bench.py's gpu_launches and per-kernel CUDA-event timing)
 KERNEL_LAUNCHES = {"lpf_select_count": 3, "lpf_scan_counts": 2, "lpf_select_fill": 2, "lpf_rpe_hidden": 1,
                    "lpf_gemm": 1, "lpf_gemm_tc": 1, "lpf_pack_weight": 1, "lpf_layernorm_act": 1, "lpf_gather_links": 1, "lpf_expand_query_links": 1, "lpf_expand_source_sweep": 1, "lpf_topk_fold": 2, "lpf_attend_fused": 1, "lpf_attend_fused_ws": 2,
-                   "lpf_gcn_spmm": 1, "lpf_gcn_layer": 1, "lpf_nz_links_fused": 2, "lpf_nz_pairs": 1, "lpf_select_compact": 2, "lpf_select_onepass": 4, "lpf_select_onepass_packed": 6, "lpf_pack_link_rows": 4, "lpf_scatter_rows": 2, "lpf_link_heads_tc": 1, "lpf_link_heads_f16": 1, "lpf_pack_weight_f16": 1}
+                   "lpf_gcn_spmm": 1, "lpf_gcn_layer": 1, "lpf_nz_links_fused": 2, "lpf_nz_pairs": 1, "lpf_select_compact": 2, "lpf_select_onepass": 4, "lpf_select_onepass_packed": 6, "lpf_pack_link_rows": 4, "lpf_scatter_rows": 2, "lpf_link_heads_tc": 1, "lpf_link_heads_f16": 1, "lpf_pack_weight_f16": 1,
+                   "lpf_gemm_wgrad": 2, "lpf_act_backward": 1, "lpf_gather_links_backward": 1,
+                   "lpf_rpe_hidden_backward": 2, "lpf_attend_backward": 1}   # (+ two counted per call: see ops.py)
 
 
 class Trace:
@@ -147,13 +164,14 @@ TRACE = None
 COUNTERS = None   # optional dict: bench.py counts CUDA-graph launches here
 
 
-def call(name, *args, meta=None, label=None):
+def call(name, *args, meta=None, label=None, launches=None):
     """Invoke an int-returning entry point; raise LpfError with lpf_last_error() on failure.  `label`: the tracer
-    files the call under name/label (two uses of one entry point that should be timed apart)."""
+    files the call under name/label (two uses of one entry point that should be timed apart).  `launches`: the kernels
+    this call launches, for entry points whose count depends on their arguments (KERNEL_LAUNCHES otherwise)."""
     lib = load()
     tr = TRACE
     if tr is not None:
-        tr.launches += KERNEL_LAUNCHES.get(name, 0)
+        tr.launches += KERNEL_LAUNCHES.get(name, 0) if launches is None else launches
         if tr.events:
             a = torch.cuda.Event(enable_timing=True)
             b = torch.cuda.Event(enable_timing=True)

@@ -111,3 +111,18 @@ def gcn_normalise(adj: CSR) -> CSR:
     dis[torch.isinf(dis)] = 0.0
     val = dis[row] * val * dis[col]
     return csr_from_coo(row, col, val, n)
+
+
+def transpose_csr(adj: CSR) -> CSR:
+    """The transpose of `adj` (the SpMM of the GCN's backward multiplies by A_hat^T): `adj` itself when it is symmetric
+    (every graph gcn_normalise builds from a symmetric adjacency), otherwise a transposed copy.  Either answer is kept on
+    the table, so it is worked out once per table."""
+    hit = adj.__dict__.get("_transpose")
+    if hit is not None:
+        return adj if hit is True else hit
+    row = torch.repeat_interleave(torch.arange(adj.n, device=adj.rowptr.device), adj.rowptr[1:] - adj.rowptr[:-1])
+    t = csr_from_coo(adj.col.to(torch.int64), row, adj.val, adj.n)
+    same = bool(torch.equal(t.rowptr, adj.rowptr) and torch.equal(t.col, adj.col) and
+                (adj.val is None or torch.equal(t.val, adj.val)))
+    adj.__dict__["_transpose"] = True if same else t
+    return adj if same else t

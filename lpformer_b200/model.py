@@ -5,11 +5,16 @@ as the reference (models/link_transformer.py, models/other_models.py, modules/la
 modules/node_encoder.py), so `from lpformer_b200 import LinkTransformer, mlp_score` drops
 into src/train's eval loops (train/testing.py:14-121) and loads reference checkpoints
 (util/utils.py:38-51) unchanged.  Every forward computation runs in the sm_100a kernels
-behind include/lpformer_b200.h; there is no PyTorch or CPU fallback, and the path is
-inference-only (no autograd through the kernels).
+behind include/lpformer_b200.h; there is no PyTorch or CPU fallback.
+
+A module in training mode with grad mode enabled builds an autograd graph through the same kernels (autograd.py; the
+backward kernels are in csrc/backward.cu), so the reference's training loop body runs at dropout 0.  In eval mode or
+under torch.no_grad() the outputs are detached, as before.  score_links / score_queries / LinkScoreStream and the plans
+are inference-only.
 """
 from __future__ import annotations
 
+import functools
 import os
 
 import math
@@ -18,9 +23,10 @@ from typing import Optional
 import torch
 import torch.nn as nn
 
+from . import autograd as AG
 from . import ops
 from ._lib import EPI_NONE, EPI_RELU, EPI_SIGMOID, LpfError
-from .graph import CSR, csr_from_sparse, gcn_normalise
+from .graph import CSR, csr_from_sparse, gcn_normalise, transpose_csr
 
 
 def _no_training(module: nn.Module, what: str):
@@ -28,6 +34,23 @@ def _no_training(module: nn.Module, what: str):
         raise NotImplementedError(
             f"lpformer_b200 is the inference path; {what} (training-time behaviour) is not implemented. "
             "Call .eval() first.")
+
+
+def _differentiable(module: nn.Module) -> bool:
+    """The training path runs when the module is in training mode and grad mode is enabled."""
+    return module.training and torch.is_grad_enabled()
+
+
+def _grad_if_training(fn):
+    """Runs `fn` with grad mode as the caller has it when the module trains (see _differentiable), under no_grad
+    otherwise (detached outputs, the inference path)."""
+    @functools.wraps(fn)
+    def wrapper(self, *args, **kwargs):
+        if _differentiable(self):
+            return fn(self, *args, **kwargs)
+        with torch.no_grad():
+            return fn(self, *args, **kwargs)
+    return wrapper
 
 
 class _GlorotLinear(nn.Module):
@@ -81,11 +104,15 @@ class MLP(nn.Module):
         if self.norm is not None:
             self.norm.reset_parameters()
 
-    @torch.no_grad()
+    @_grad_if_training
     def forward(self, x, out=None):
         _no_training(self, "dropout" if self.dropout > 0 else "")
         lead = x.shape[:-1]
         x = x.reshape(-1, x.shape[-1])
+        if torch.is_grad_enabled():
+            AG.require_training_inputs(x)
+            x = AG.MLPFunction.apply(x, self.norm is not None, self.sigmoid, *AG.mlp_params(self.linears, self.norm))
+            return x.reshape(*lead, x.shape[-1]).squeeze(-1)
         for lin in list(self.linears)[:-1]:
             if self.norm is not None:
                 x = ops.linear(x, lin.weight, lin.bias)
@@ -117,10 +144,13 @@ class mlp_score(nn.Module):
         for lin in self.lins:
             lin.reset_parameters()
 
-    @torch.no_grad()
+    @_grad_if_training
     def forward(self, x, return_logits=False):
         _no_training(self, "dropout" if self.dropout > 0 else "")
         x = x.reshape(-1, x.shape[-1])
+        if torch.is_grad_enabled():
+            AG.require_training_inputs(x)
+            return AG.MLPFunction.apply(x, False, not return_logits, *AG.mlp_params(self.lins, None)).squeeze(-1)
         for lin in list(self.lins)[:-1]:
             x = ops.linear(x, lin.weight, lin.bias, epilogue=EPI_RELU)
         last = self.lins[-1]
@@ -182,13 +212,24 @@ class GCN(nn.Module):
         for conv in self.convs:
             conv.reset_parameters()
 
-    @torch.no_grad()
+    @_grad_if_training
     def forward(self, x, adj_norm: CSR, final_norm=None):
         """reference :61-76.  Per layer one contraction (x W^T) and ONE launch for the rest (SpMM + bias + LayerNorm +
         ReLU + residual, ops.gcn_layer); final_norm = (weight, bias) of a LayerNorm applied to the last layer's output
         in the same launch (LinkTransformer.gnn_norm)."""
         _no_training(self, "dropout" if self.dropout > 0 else "")
         last = len(self.convs) - 1
+        if torch.is_grad_enabled():
+            AG.require_training_inputs(x)
+            adj_t = transpose_csr(adj_norm)
+            for i, conv in enumerate(self.convs):
+                ln = self.lns[i] if self.lns is not None else None
+                ln2 = final_norm if i == last else None
+                x = AG.GCNLayerFunction.apply(x, conv.lin.weight, conv.bias, None if ln is None else ln.weight,
+                                              None if ln is None else ln.bias, None if ln2 is None else ln2[0],
+                                              None if ln2 is None else ln2[1], adj_norm, adj_t, self.relu,
+                                              bool(self.residual and x.shape[-1] == conv.lin.weight.shape[0]))
+            return x
         for i, conv in enumerate(self.convs):
             xw = ops.linear(x, conv.lin.weight)
             ln = self.lns[i] if self.lns is not None else None
@@ -212,7 +253,7 @@ class NodeEncoder(nn.Module):
                                cached=train_args.get("gcn_cache"), residual=train_args["residual"],
                                layer_norm=train_args["layer_norm"], relu=train_args["relu"])
 
-    @torch.no_grad()
+    @_grad_if_training
     def forward(self, features, adj_norm: CSR, test_set=False, final_norm=None):
         _no_training(self, "feature dropout" if self.feat_drop > 0 else "")
         return self.gnn_encoder(features, adj_norm, final_norm=final_norm)
@@ -454,7 +495,7 @@ class LinkTransformer(nn.Module):
             return self._kv_cache[1]
         d = self.dim
         kvs = [ops.linear(X_node, layer.att.lin_r.weight[:, :d]) for layer in self.att_layers]
-        self._kv_cache = (key, kvs, X_node)   # keep X_node alive so the pointer key stays valid
+        self._kv_cache = (key, kvs, X_node.detach())   # keep X_node alive so the pointer key stays valid
         return kvs
 
     def _prime_kv(self, X_node, kvs):
@@ -464,11 +505,18 @@ class LinkTransformer(nn.Module):
         self._kv_cache = (key, kvs, X_node)
 
     # ------------------------------------------------------------------ reference API
-    @torch.no_grad()
+    @_grad_if_training
     def forward(self, batch, adj_prop=None, adj_mask=None, test_set=False, return_weights=False):
         """reference :82-107."""
         batch = ops.links_tensor(batch, self._dev())
         X_node = self.propagate(adj_prop, test_set)
+        if torch.is_grad_enabled():
+            # both halves carry gradients: each is built by its own Function, then joined by the row-copy kernel
+            xprod = AG.GatherLinksFunction.apply(self._check_x(X_node), batch, None, True)
+            el = self.elementwise_lin(xprod)
+            pw, att_weights = self.calc_pairwise(batch, X_node, test_set, adj_mask=adj_mask, return_weights=return_weights)
+            feats = AG.ConcatFunction.apply(el, pw)
+            return feats if not return_weights else (feats, att_weights)
         feats = torch.empty((batch.shape[1], 2 * self.dim), dtype=torch.float32, device=self._dev())
         _, xprod = ops.gather_links(batch, X_node, want_sum=False, want_prod=True)
         self.elementwise_lin(xprod, out=feats[:, : self.dim])
@@ -476,7 +524,7 @@ class LinkTransformer(nn.Module):
                                             out=feats[:, self.dim:])
         return feats if not return_weights else (feats, att_weights)
 
-    @torch.no_grad()
+    @_grad_if_training
     def propagate(self, adj=None, test_set=False):
         """reference :110-129 — GCN over the whole graph, then gnn_norm."""
         if adj is None:
@@ -486,7 +534,9 @@ class LinkTransformer(nn.Module):
         x = self.data["x"]
         if "emb" in self.data:
             x = self.data["emb"](x)
-        x = x.detach().to(self._dev(), torch.float32)
+        x = x.to(self._dev(), torch.float32)
+        if not torch.is_grad_enabled():
+            x = x.detach()
         # (gnn_norm rides in the epilogue of the last GCN layer's launch)
         return self.node_encoder(x, adj_norm, test_set, final_norm=(self.gnn_norm.weight, self.gnn_norm.bias))
 
@@ -521,7 +571,7 @@ class LinkTransformer(nn.Module):
         far = ops.select(batch, stored, self.get_ppr(test_set), *th, "all", want_link=want_link)
         return ops.merge_selections(near, far)
 
-    @torch.no_grad()
+    @_grad_if_training
     def calc_pairwise(self, batch, X_node, test_set=False, adj_mask=None, return_weights=False, out=None):
         """reference :132-178.  Returns (pairwise feats [BS, dim], att_weights [2,S] or None).
 
@@ -534,6 +584,8 @@ class LinkTransformer(nn.Module):
         bs = batch.shape[1]
         sel = self._select(batch, test_set, adj_mask, want_link=return_weights)
         nnz = sel.nz.numel()
+        if torch.is_grad_enabled():
+            return self._pairwise_differentiable(batch, X_node, sel, return_weights)
         if return_weights or nnz == bs or bs == 0:
             pw, alpha = self._pairwise_rows(batch, X_node, sel, None, out=out, want_alpha=return_weights)
         else:
@@ -549,14 +601,52 @@ class LinkTransformer(nn.Module):
     def _check_x(self, X_node):
         if not X_node.is_cuda:
             raise LpfError("X_node must be a CUDA tensor")
-        X_node = X_node.detach()
+        if not torch.is_grad_enabled():
+            X_node = X_node.detach()
         if X_node.dtype != torch.float32 or X_node.stride(-1) != 1:
             X_node = X_node.float().contiguous()
         return X_node
 
+    def _pairwise_differentiable(self, batch, X_node, sel, return_weights):
+        """calc_pairwise with autograd (training mode): the empty-set links share one pairwise row, built through the
+        attention bias -> LayerNorm -> pairwise_lin chain once, whose gradient is the sum over those links."""
+        bs, nnz = sel.bs, sel.nz.numel()
+        params = AG.pairwise_params(self)
+        alpha = None
+        if return_weights or nnz == bs or bs == 0:
+            res = AG.PairwiseFunction.apply(X_node, self, batch, sel, None, return_weights, *params)
+            feats, alpha = res if return_weights else (res, None)
+            pw = self.pairwise_lin(feats)
+        else:
+            rows = None
+            if nnz > 0:
+                rows = self.pairwise_lin(AG.PairwiseFunction.apply(X_node, self, batch, sel, sel.nz, False, *params))
+            pw = AG.ScatterFillFunction.apply(rows, self._pw_const_differentiable(X_node, params), sel.nz, bs)
+        att_weights = torch.stack((sel.link.float(), alpha)) if return_weights else None
+        return pw, att_weights
+
+    def _empty_selection(self):
+        dev = self._dev()
+        return ops.Selection(self.mask, 1, torch.zeros(4, dtype=torch.int64, device=dev),
+                             torch.empty(0, dtype=torch.int32, device=dev), torch.empty(0, device=dev),
+                             torch.empty(0, device=dev), None, (0, 0, 0, 0), torch.empty(0, dtype=torch.int32, device=dev))
+
+    def _pw_const_differentiable(self, X_node, params):
+        """[1, dim] pairwise row of a link with empty node sets, with its autograd graph (built per call: a cached row
+        would carry a graph that the first backward frees)."""
+        empty = torch.zeros((2, 1), dtype=torch.int64, device=self._dev())
+        return self.pairwise_lin(AG.PairwiseFunction.apply(X_node, self, empty, self._empty_selection(), None, False,
+                                                           *params))
+
     def _pairwise_rows(self, batch, X_node, sel, idx, out=None, want_alpha=False):
         """RPE -> attention layers -> counts -> pairwise_lin for the batch positions in idx (all links when None).
         Returns ([n, dim] rows in idx order, per-pair attention weights or None)."""
+        feats, alpha, _ = self._attention_stack(batch, X_node, sel, idx, want_alpha)
+        return self.pairwise_lin(feats, out=out), alpha
+
+    def _attention_stack(self, batch, X_node, sel, idx, want_alpha=False, save=False):
+        """RPE -> attention layers -> counts for the batch positions in idx (all links when None): ([n, H*C +
+        count_dim] rows in idx order, per-pair attention weights or None, and with save=True what the backward reads)."""
         dev = self._dev()
         d, H = self.dim, self.num_heads
         n = sel.bs if idx is None else idx.numel()
@@ -599,6 +689,8 @@ class LinkTransformer(nn.Module):
         xsum, _ = ops.gather_links(batch, X_node, want_sum=True, want_prod=False, idx=idx)   # e1 + e2 of layer 0
         alpha = torch.empty(S, dtype=torch.float32, device=dev) if want_alpha else None
         feats = None
+        st = {"csel": csel, "r_map": r_map, "hsum": hsum, "h0": h0 if r_map is not None else None, "kvs": kvs,
+              "derived": derived, "Q": [], "R": [], "r_const": [], "feats_in": []} if save else None
         for l, layer in enumerate(self.att_layers):
             att = layer.att
             C = att.out_channels
@@ -618,11 +710,16 @@ class LinkTransformer(nn.Module):
                 if r_map is not None:
                     ops.linear(h0[t:t + 1], m, c, out=r_const[t:t + 1])
             width = HC + (self.count_dim if last else 0)
+            if save:
+                st["Q"].append(Q)
+                st["R"].append(R)
+                st["r_const"].append(r_const)
+                st["feats_in"].append(xsum if l == 0 else feats)
             feats = torch.empty((n, width), dtype=torch.float32, device=dev)
             ops.attend(sel, kvs[l], R, Q, att.att, att.bias, layer.post_att_norm.weight, layer.post_att_norm.bias,
                        H, C, write_counts=last, out=feats, alpha_out=alpha if last else None, idx=idx,
                        r_map=r_map, r_const=r_const)
-        return self.pairwise_lin(feats, out=out), alpha
+        return feats, alpha, st
 
     def _node_tables(self, X_node, kv):
         """(X, KV) as the plan's kernels read them: the fp32 tensors, or bf16 copies built once per X_node."""
@@ -639,11 +736,8 @@ class LinkTransformer(nn.Module):
         if self._pw_const_cache is not None and self._pw_const_cache[0] == key:
             return self._pw_const_cache[1]
         dev = self._dev()
-        empty = ops.Selection(self.mask, 1, torch.zeros(4, dtype=torch.int64, device=dev),
-                              torch.empty(0, dtype=torch.int32, device=dev), torch.empty(0, device=dev),
-                              torch.empty(0, device=dev), None, (0, 0, 0, 0),
-                              torch.empty(0, dtype=torch.int32, device=dev))
-        row = self._pairwise_rows(torch.zeros((2, 1), dtype=torch.int64, device=dev), X_node, empty, None)[0]
+        row = self._pairwise_rows(torch.zeros((2, 1), dtype=torch.int64, device=dev), X_node, self._empty_selection(),
+                                  None)[0]
         self._pw_const_cache = (key, row)
         return row
 

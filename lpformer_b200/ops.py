@@ -231,6 +231,7 @@ def merge_selections(near: Selection, far: Selection) -> Selection:
 def drop_packed_weights():
     """Forgets every cached tensor-core weight image (LinkTransformer.invalidate_weights)."""
     _PACKED.clear()
+    _PACKED_T.clear()
 
 
 def links_tensor(batch, device) -> torch.Tensor:
@@ -560,3 +561,161 @@ def gcn_spmm(adj: CSR, XW, bias, out=None, row0=0, rows=None):
     call("lpf_gcn_spmm", ptr(adj.rowptr), ptr(adj.col), ptr(adj.val), row0, rows, ptr(XW), XW.stride(0), ptr(bias), d,
          ptr(out), out.stride(0), stream())
     return out
+
+
+# ---------------------------------------------------------------------------------------------- backward (backward.cu)
+def _workspace(nbytes, device):
+    if nbytes < 0:
+        raise ValueError("bad workspace arguments")
+    return torch.empty(max(1, (nbytes + 15) // 16 * 4), dtype=torch.float32, device=device)
+
+
+def layernorm_act_backward(x, weight, bias, dy, relu=False, dx=None, accumulate_dx=False, dweight=None, dbias=None,
+                           accumulate_param=False, n=None):
+    """Gradients of y = act(LN(x[:, :n])) (lpf_layernorm_act) from the saved pre-norm rows x: dx (written, or added with
+    accumulate_dx) and, with weight, dweight / dbias (written, or added with accumulate_param).  Returns dx."""
+    require_cuda(x, weight, bias, dy, dx, dweight, dbias)
+    x, dy = _rowmajor(x), _rowmajor(dy)
+    rows = x.shape[0]
+    n = x.shape[1] if n is None else n
+    if dx is None:
+        dx = torch.empty((rows, n), dtype=torch.float32, device=x.device)
+    ws = None
+    if weight is not None:
+        if dweight is None or dbias is None:
+            raise ValueError("layernorm_act_backward: dweight and dbias are needed with weight")
+        ws = _workspace(_lib.load().lpf_layernorm_act_backward_workspace_bytes(rows, n), x.device)
+    call("lpf_layernorm_act_backward", ptr(x), x.stride(0), ptr(weight), ptr(bias), int(relu), ptr(dy), dy.stride(0),
+         ptr(dx), dx.stride(0), int(accumulate_dx), ptr(dweight), ptr(dbias), int(accumulate_param), rows, n, ptr(ws),
+         0 if ws is None else 4 * ws.numel(), stream(), meta=(rows, n),
+         launches=0 if rows == 0 else (3 if weight is not None else 1))      # (with weight: + two reductions)
+    return dx
+
+
+def gemm_wgrad(A, dY, dW=None, db=None, accumulate=False):
+    """dW (+)= dY^T A and db (+)= the column sums of dY (lpf_gemm_wgrad); A may be None when only db is wanted."""
+    require_cuda(A, dY, dW, db)
+    dY = _rowmajor(dY)
+    M, N = dY.shape
+    K = 1
+    if dW is not None:
+        A = _rowmajor(A)
+        K = A.shape[1]
+        if A.shape[0] != M or tuple(dW.shape) != (N, K) or dW.stride(1) != 1:
+            raise ValueError(f"gemm_wgrad: A {list(A.shape)}, dY {list(dY.shape)}, dW {list(dW.shape)}")
+    ws = _workspace(_lib.load().lpf_gemm_wgrad_workspace_bytes(M, N, K), dY.device)
+    call("lpf_gemm_wgrad", ptr(A) if dW is not None else None, A.stride(0) if dW is not None else K, ptr(dY),
+         dY.stride(0) if M > 0 else N, M, N, K, ptr(dW), dW.stride(0) if dW is not None else K, ptr(db), int(accumulate),
+         ptr(ws), 4 * ws.numel(), stream(), meta=(M, N, K))
+
+
+_PACKED_T = {}        # transposed weight images of linear_dgrad: (data_ptr, shape, stride, k0) -> (version, image, weight)
+
+
+def linear_dgrad(dY, W, out=None, cache=True):
+    """dX[M, K] = dY[M, N] @ W[N, K] on the tensor cores (lpf_gemm_tc on the packed transpose of W, in chunks of 256
+    output columns).  cache=False for a W built for this call only: its image is not kept."""
+    require_cuda(dY, W, out)
+    dY = _rowmajor(dY)
+    M, N = dY.shape
+    K = W.shape[1]
+    if W.shape[0] != N:
+        raise ValueError(f"linear_dgrad: dY is [{M},{N}] but W is {list(W.shape)}")
+    if out is None:
+        out = torch.empty((M, K), dtype=torch.float32, device=dY.device)
+    for k0 in range(0, K, 256):
+        k1 = min(K, k0 + 256)
+        key = (W.data_ptr(), tuple(W.shape), W.stride(0), W.device.index, k0)
+        hit = _PACKED_T.get(key) if cache else None
+        if hit is None or hit[0] != W._version or hit[2] is not W:     # (an optimizer step replaces the entry)
+            Wt = W.detach()[:, k0:k1].t().contiguous()
+            nbytes = _lib.load().lpf_pack_weight_bytes(k1 - k0, N)
+            img = torch.empty(nbytes // 4, dtype=torch.float32, device=W.device)
+            call("lpf_pack_weight", ptr(Wt), Wt.stride(0), k1 - k0, N, ptr(img), stream())
+            hit = (W._version, img, W)
+            if cache:
+                if len(_PACKED_T) > 512:
+                    _PACKED_T.clear()
+                _PACKED_T[key] = hit
+        o = out[:, k0:k1]
+        call("lpf_gemm_tc", ptr(dY), dY.stride(0), ptr(hit[1]), None, 1.0, ptr(o), o.stride(0) if M > 0 else k1 - k0, M,
+             k1 - k0, N, EPI_NONE, None, stream(), meta=(M, k1 - k0, N))
+    return out
+
+
+def act_backward(y, dy, act, out=None):
+    """dx = dy [y > 0] (EPI_RELU) or dy y (1 - y) (EPI_SIGMOID) from the saved output y."""
+    require_cuda(y, dy, out)
+    y, dy = _rowmajor(y), _rowmajor(dy)
+    rows, n = y.shape
+    if out is None:
+        out = torch.empty((rows, n), dtype=torch.float32, device=y.device)
+    call("lpf_act_backward", ptr(y), y.stride(0), ptr(dy), dy.stride(0), ptr(out), out.stride(0), rows, n, act, stream())
+    return out
+
+
+def gather_links_backward(links, X, dX, dsum=None, dprod=None, idx=None):
+    """dX[a] += dsum + dprod X[b], dX[b] += dsum + dprod X[a] for every link (or the positions in idx)."""
+    require_cuda(links, X, dX, dsum, dprod, idx)
+    X = _rowmajor(X)
+    bs, d = links.shape[1], X.shape[1]
+    n = bs if idx is None else idx.numel()
+    dsum = None if dsum is None else _rowmajor(dsum)
+    dprod = None if dprod is None else _rowmajor(dprod)
+    call("lpf_gather_links_backward", ptr(links), bs, ptr(idx), n, ptr(X), X.stride(0), d, ptr(dsum),
+         dsum.stride(0) if dsum is not None else 0, ptr(dprod), dprod.stride(0) if dprod is not None else 0, ptr(dX),
+         dX.stride(0), stream(), meta=(n, d))
+    return dX
+
+
+def scatter_rows_backward(dG, idx, want_src=True):
+    """(d src [n, d] or None, d fill_row [d]) of scatter_rows(src, idx, dst, fill_row)."""
+    require_cuda(dG, idx)
+    dG = _rowmajor(dG)
+    rows, d = dG.shape
+    n = 0 if idx is None else idx.numel()
+    dsrc = torch.empty((n, d), dtype=torch.float32, device=dG.device) if want_src and n > 0 else None
+    dfill = torch.empty(d, dtype=torch.float32, device=dG.device)
+    ws = _workspace(_lib.load().lpf_scatter_rows_backward_workspace_bytes(rows, d), dG.device)
+    call("lpf_scatter_rows_backward", ptr(dG), dG.stride(0), rows, d, ptr(idx), n, ptr(dsrc), d, ptr(dfill), ptr(ws),
+         4 * ws.numel(), stream(), meta=(rows, d), launches=(1 if n > 0 else 0) + 2)   # gather + masked sum + reduction
+    return dsrc, dfill
+
+
+def rpe_hidden_backward(src_ppr, tgt_ppr, r0, r1, w1, b1, ln_w, ln_b, dh, grads, accumulate):
+    """Adds (or writes) the gradients of one PPR encoder's first Linear + LayerNorm from dh = d hsum[r0:r1] (rows of dh
+    in pair order).  grads: (dw1 [d, 2], db1, dln_w, dln_b)."""
+    require_cuda(src_ppr, tgt_ppr, w1, dh, *grads)
+    d = w1.shape[0]
+    rows = r1 - r0
+    dh = None if rows == 0 else _rowmajor(dh)
+    ws = _workspace(_lib.load().lpf_rpe_hidden_backward_workspace_bytes(rows, d), w1.device)
+    call("lpf_rpe_hidden_backward", ptr(src_ppr), ptr(tgt_ppr), r0, rows, ptr(w1), ptr(b1), ptr(ln_w), ptr(ln_b), d,
+         ptr(dh), dh.stride(0) if rows > 0 else d, *[ptr(g) for g in grads], int(accumulate), ptr(ws), 4 * ws.numel(),
+         stream(), meta=(rows, d))
+
+
+def attend_backward(sel: Selection, KV, R, Q, att, bias, ln_w, ln_b, heads, ch, dY, dKV, idx=None, r_map=None,
+                    r_const=None, dR=None, dR_const=None):
+    """Backward of attend() (lpf_attend_backward): writes dR [rows of R, HC] (needed when R has rows), adds into
+    dR_const [3, HC] (needed with r_map) and dKV [N, HC], and returns (dQ [n, HC], link_rows [n, 4 HC])."""
+    require_cuda(KV, R, Q, dY, dKV, idx, r_map, r_const, dR, dR_const)
+    n = sel.bs if idx is None else idx.numel()
+    HC = heads * ch
+    dev = KV.device
+    dY = _rowmajor(dY)
+    if R is None or R.shape[0] == 0:
+        dR = None
+    elif dR is None or dR.shape != R.shape or dR.stride(1) != 1:
+        raise ValueError("attend_backward: dR must be a row-major table shaped like R")
+    if (r_map is None) != (dR_const is None):
+        raise ValueError("attend_backward: dR_const goes with r_map")
+    dRc = dR_const
+    dQ = torch.empty((n, HC), dtype=torch.float32, device=dev)
+    rows = torch.empty((n, 4 * HC), dtype=torch.float32, device=dev)
+    call("lpf_attend_backward", ptr(sel.ptr), sel.bs, ptr(idx), n, ptr(sel.node), ptr(KV), KV.stride(0),
+         ptr(R) if dR is not None else None, R.stride(0) if dR is not None else HC, ptr(r_map), ptr(r_const), ptr(Q),
+         Q.stride(0), ptr(att), ptr(bias), ptr(ln_w), ptr(ln_b), heads, ch, ptr(dY), dY.stride(0), ptr(dR),
+         dR.stride(0) if dR is not None else HC, ptr(dRc), ptr(dQ), HC, ptr(dKV), dKV.stride(0), ptr(rows), stream(),
+         meta=(n, sel.total, HC))
+    return dQ, rows
