@@ -488,7 +488,7 @@ void* lpf_ppr_push_host(const int64_t* indptr_host, const int32_t* indices_host,
 int lpf_ppr_push_host_fetch(void* handle, int64_t* rowptr_host, int32_t* col_host, float* val_host);
 
 /* ------------------------------------------------------------------------- *
- * Backward pass (training at dropout 0): the gradients of the host-sized forward with respect to the reference's
+ * Backward pass (training, dropout included: see "Dropout" below): the gradients of the host-sized forward with respect to the reference's
  * parameters and to X_node.  Parameter gradients are reduced deterministically through a caller-owned workspace
  * (size from the matching *_workspace_bytes; -1 = bad arguments); `accumulate` != 0 adds into the outputs instead of
  * overwriting them.  Scatters into node-indexed tables (dX, dKV) are fp32 atomic adds into zero-initialised tables.
@@ -544,6 +544,54 @@ int lpf_attend_backward(const int64_t* ptr, int64_t bs, const int32_t* idx, int6
                         const float* ln_w, const float* ln_b, int32_t heads, int32_t ch, const float* dY,
                         int64_t ld_dy, float* dR, int64_t ld_dr, float* dR_const, float* dQ, int64_t ld_dq,
                         float* dKV, int64_t ld_dkv, float* link_rows, void* stream);
+
+/* ------------------------------------------------------------------------- *
+ * Dropout (training mode; F.dropout semantics: each element is zeroed with probability p, kept elements are scaled
+ * by 1 / (1 - p); p outside [0, 1] is LPF_ERR_INVALID).  The sites and their `site` numbers (lpformer_b200/ops.py):
+ * the GCN input features (1), node dropout of the selected pairs (2), GCN layer l (16 + l, after the activation),
+ * attention layer l's output (32 + l), hidden layer i of an MLP / mlp_score (48 + i).
+ *
+ * Random numbers: counter-based Philox4x32-10 with key = the 64-bit seed (low word, high word) and counter =
+ * (col >> 2, row low word, row high word, site); element (row, col) reads word col & 3.  `row` is the global row (the
+ * node id of node tables, the batch position of link tables, the pair index of node dropout), so a mask does not depend
+ * on row sharding (row0), index subsets or the launch shape.  Keep rule: the word u keeps the element iff
+ * u >= floor(p 2^32); a kept element becomes x * fp32(1 / (1 - p)) (exactly that product), a dropped one 0.
+ * The seed is read from device memory (`seed`: one uint64), so a seed drawn on the device needs no host sync.  Masks
+ * are never stored: the backward regenerates them from the seed.
+ *
+ * lpf_dropout: Y[r, :n] = X[r, :n] * mask(row0 + r) / (1 - p) for rows [0, rows); X == Y is allowed (in place).  The
+ *   forward of the feature, attention-output and MLP sites, the backward of every site (on dY), and on a table of ones
+ *   the mask itself (mask / (1 - p)).
+ * lpf_gcn_layer_dropout: lpf_gcn_layer with dropout between the activation and the residual:
+ *   Y = LN2(residual + drop(act(LN1(A_hat XW + bias)))), mask row = node id.  (The reference's order conv -> LN ->
+ *   dropout -> ReLU gives the same values: relu(m z / (1 - p)) == m relu(z) / (1 - p) exactly in fp32.)
+ * lpf_layernorm_act_dropout: Y = residual + drop(act(LN(X))) (lpf_layernorm_act with the same dropout; mask row =
+ *   row0 + r): the GCN backward's recompute of the rows that enter gnn_norm.
+ * lpf_drop_pairs_count / lpf_drop_pairs_fill: node dropout (reference compute_node_mask -> drop_pairwise) of a
+ *   selection (ptr [3 bs + 1], node / src_ppr / tgt_ppr / link [S], type-major, (link, node)-sorted): keeps exactly K
+ *   pairs, a uniform K-subset (pair i's key: 64 Philox bits of (seed, site, row i, col 0) with its low
+ *   ceil(log2 S) bits replaced by i; the K smallest keys are kept).  _count writes the kept pairs per (type, link)
+ *   segment into counts [3 bs] (scan them with lpf_scan_counts into ptr_out, and lpf_select_compact gives the non-empty
+ *   links and the new type bounds); _fill copies the kept pairs in order to ptr_out's positions (link / link_out may
+ *   both be NULL).  The workspace (lpf_drop_pairs_workspace_bytes) carries the threshold from _count to _fill.
+ * ------------------------------------------------------------------------- */
+int lpf_dropout(const float* X, int64_t ldx, float* Y, int64_t ldy, int64_t rows, int32_t n, int64_t row0,
+                const uint64_t* seed, int32_t site, double p, void* stream);
+int lpf_gcn_layer_dropout(const int64_t* rowptr, const int32_t* col, const float* val, int64_t row0, int64_t rows,
+                          const float* XW, int64_t ld_xw, const float* bias, int32_t d, const float* ln_w,
+                          const float* ln_b, int relu, const uint64_t* seed, int32_t site, double p,
+                          const float* residual, int64_t ld_res, const float* ln2_w, const float* ln2_b, float* Y,
+                          int64_t ldy, void* stream);
+int lpf_layernorm_act_dropout(const float* X, int64_t ldx, const float* gamma, const float* beta, int relu,
+                              int64_t row0, const uint64_t* seed, int32_t site, double p, const float* residual,
+                              int64_t ldr, float* Y, int64_t ldy, int64_t rows, int32_t n, void* stream);
+int64_t lpf_drop_pairs_workspace_bytes(void);
+int lpf_drop_pairs_count(const int64_t* ptr, int64_t bs, int64_t S, int64_t K, const uint64_t* seed, int32_t site,
+                         int32_t* counts, void* workspace, int64_t workspace_bytes, void* stream);
+int lpf_drop_pairs_fill(const int64_t* ptr, int64_t bs, const int32_t* node, const float* src_ppr,
+                        const float* tgt_ppr, const int32_t* link, int64_t S, const uint64_t* seed, int32_t site,
+                        const void* workspace, const int64_t* ptr_out, int32_t* node_out, float* src_out,
+                        float* tgt_out, int32_t* link_out, void* stream);
 
 #ifdef __cplusplus
 }

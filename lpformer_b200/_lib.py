@@ -18,6 +18,7 @@ EPI_NONE, EPI_RELU, EPI_SIGMOID = 0, 1, 2
 ALGO_GENERIC, ALGO_INTERSECT8, ALGO_INTERSECT32, ALGO_PACKED = 0, 1, 2, 3
 
 _p, _i64, _i32, _f32, _int = C.c_void_p, C.c_int64, C.c_int32, C.c_float, C.c_int
+_f64 = C.c_double
 
 # name -> (restype, argtypes); mirrors include/lpformer_b200.h line by line
 SIGNATURES = {
@@ -92,6 +93,15 @@ SIGNATURES = {
                                        _p]),
     "lpf_attend_backward": (_int, [_p, _i64, _p, _i64, _p, _p, _i64, _p, _i64, _p, _p, _p, _i64, _p, _p, _p, _p, _i32,
                                    _i32, _p, _i64, _p, _i64, _p, _p, _i64, _p, _i64, _p, _p]),
+    # dropout (csrc/dropout.cu, spmm.cu, dense.cu)
+    "lpf_dropout": (_int, [_p, _i64, _p, _i64, _i64, _i32, _i64, _p, _i32, _f64, _p]),
+    "lpf_gcn_layer_dropout": (_int, [_p, _p, _p, _i64, _i64, _p, _i64, _p, _i32, _p, _p, _int, _p, _i32, _f64, _p, _i64,
+                                     _p, _p, _p, _i64, _p]),
+    "lpf_layernorm_act_dropout": (_int, [_p, _i64, _p, _p, _int, _i64, _p, _i32, _f64, _p, _i64, _p, _i64, _i64, _i32,
+                                         _p]),
+    "lpf_drop_pairs_workspace_bytes": (_i64, []),
+    "lpf_drop_pairs_count": (_int, [_p, _i64, _i64, _i64, _p, _i32, _p, _p, _i64, _p]),
+    "lpf_drop_pairs_fill": (_int, [_p, _i64, _p, _p, _p, _p, _i64, _p, _i32, _p, _p, _p, _p, _p, _p, _p]),
 }
 
 
@@ -139,7 +149,9 @@ KERNEL_LAUNCHES = {"lpf_select_count": 3, "lpf_scan_counts": 2, "lpf_select_fill
                    "lpf_gemm": 1, "lpf_gemm_tc": 1, "lpf_pack_weight": 1, "lpf_layernorm_act": 1, "lpf_gather_links": 1, "lpf_expand_query_links": 1, "lpf_expand_source_sweep": 1, "lpf_topk_fold": 2, "lpf_attend_fused": 1, "lpf_attend_fused_ws": 2,
                    "lpf_gcn_spmm": 1, "lpf_gcn_layer": 1, "lpf_nz_links_fused": 2, "lpf_nz_pairs": 1, "lpf_select_compact": 2, "lpf_select_onepass": 4, "lpf_select_onepass_packed": 6, "lpf_pack_link_rows": 4, "lpf_scatter_rows": 2, "lpf_link_heads_tc": 1, "lpf_link_heads_f16": 1, "lpf_pack_weight_f16": 1,
                    "lpf_gemm_wgrad": 2, "lpf_act_backward": 1, "lpf_gather_links_backward": 1,
-                   "lpf_rpe_hidden_backward": 2, "lpf_attend_backward": 1}   # (+ two counted per call: see ops.py)
+                   "lpf_rpe_hidden_backward": 2, "lpf_attend_backward": 1,
+                   "lpf_dropout": 1, "lpf_gcn_layer_dropout": 1, "lpf_layernorm_act_dropout": 1, "lpf_drop_pairs_count": 18,
+                   "lpf_drop_pairs_fill": 1}   # (+ two counted per call: see ops.py)
 
 
 class Trace:

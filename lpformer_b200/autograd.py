@@ -1,7 +1,8 @@
-"""autograd Functions of the training path (dropout 0): every forward runs the same kernels as the inference path, so
-the values are bit-identical to eval mode, and every backward runs the kernels of csrc/backward.cu.  PyTorch does the
-plumbing only: allocation, weight-sized products (the gradients of the folded weights mapped back onto the reference's
-parameters) and the autograd graph.
+"""autograd Functions of the training path: at dropout 0 every forward runs the same kernels as the inference path, so
+the values are bit-identical to eval mode, and every backward runs the kernels of csrc/backward.cu.  With dropout the
+forwards apply the masks of csrc/dropout.cu (seed and site per call) and the backwards regenerate them from the seed:
+no mask is stored.  PyTorch does the plumbing only: allocation, weight-sized products (the gradients of the folded
+weights mapped back onto the reference's parameters) and the autograd graph.
 
 Used by lpformer_b200.model when a module is in training mode and grad mode is enabled."""
 from __future__ import annotations
@@ -10,6 +11,7 @@ import torch
 
 from . import ops
 from ._lib import EPI_NONE, EPI_RELU, EPI_SIGMOID, require_cuda
+from .ops import _rowmajor
 
 
 def _zeros_like(p):
@@ -18,17 +20,18 @@ def _zeros_like(p):
 
 # ---------------------------------------------------------------------------------------------------------------- MLP
 class MLPFunction(torch.autograd.Function):
-    """Linear -> [LayerNorm] -> ReLU ... -> Linear [-> sigmoid] (MLP.forward / mlp_score.forward) over the rows of x.
-    params: (W_0, b_0, ..., W_L, b_L[, norm.weight, norm.bias]) — the LayerNorm is shared by every hidden layer."""
+    """Linear -> [LayerNorm] -> ReLU [-> dropout] ... -> Linear [-> sigmoid] (MLP.forward / mlp_score.forward) over the
+    rows of x.  params: (W_0, b_0, ..., W_L, b_L[, norm.weight, norm.bias]) — the LayerNorm is shared by every hidden
+    layer.  p > 0: hidden layer i is dropped with the mask (seed, SITE_MLP + i), row = row of x."""
 
     @staticmethod
-    def forward(ctx, x, norm, sigmoid, *params):
+    def forward(ctx, x, norm, sigmoid, p, seed, *params):
         n_lin = (len(params) - (2 if norm else 0)) // 2
         lins = [(params[2 * i], params[2 * i + 1]) for i in range(n_lin)]
         g, b = (params[-2], params[-1]) if norm else (None, None)
         inputs, pre = [], []
         h = x
-        for W, bias in lins[:-1]:
+        for i, (W, bias) in enumerate(lins[:-1]):
             inputs.append(h)
             if norm:
                 z = ops.linear(h, W, bias)
@@ -36,11 +39,13 @@ class MLPFunction(torch.autograd.Function):
                 h = ops.layernorm_act(z, g, b, relu=True)
             else:
                 h = ops.linear(h, W, bias, epilogue=EPI_RELU)
-                pre.append(h)
+                pre.append(h)      # (dropped in place below: [h > 0] still selects the gradient, see backward)
+            if p > 0:
+                ops.dropout(h, p, seed, ops.SITE_MLP + i, out=h)   # the dropped rows feed the next layer and its dW
         inputs.append(h)
         W, bias = lins[-1]
         out = ops.linear(h, W, bias, epilogue=EPI_SIGMOID if sigmoid else EPI_NONE)
-        ctx.norm, ctx.sigmoid, ctx.n_lin = norm, sigmoid, n_lin
+        ctx.norm, ctx.sigmoid, ctx.n_lin, ctx.p, ctx.seed = norm, sigmoid, n_lin, p, seed
         ctx.save_for_backward(out, *inputs, *pre, *params)
         return out
 
@@ -65,6 +70,9 @@ class MLPFunction(torch.autograd.Function):
             if i == 0 and not ctx.needs_input_grad[0]:
                 break
             dh = ops.linear_dgrad(dy, W)
+            if i > 0 and ctx.p > 0:
+                # the mask zeroes dh where the ReLU / LayerNorm output was dropped, so their backward needs nothing else
+                ops.dropout(dh, ctx.p, ctx.seed, ops.SITE_MLP + i - 1, out=dh)
             if i == 0:
                 dx = dh
             elif ctx.norm:
@@ -74,7 +82,7 @@ class MLPFunction(torch.autograd.Function):
                 dy = ops.act_backward(pre[i - 1], dh, EPI_RELU)
         if ctx.norm:
             grads[-2], grads[-1] = dn
-        return (dx, None, None, *grads)
+        return (dx, None, None, None, None, *grads)
 
 
 def mlp_params(lins, norm):
@@ -88,16 +96,17 @@ def mlp_params(lins, norm):
 
 # ---------------------------------------------------------------------------------------------------------- GCN layer
 class GCNLayerFunction(torch.autograd.Function):
-    """One GCN layer (GCN.forward, reference models/other_models.py:61-76): out = LN2(res + act(LN(A_hat x W^T + b))),
-    where res = x when `residual`; LN / LN2 optional.  adj_t: the transpose of adj (adj itself when symmetric)."""
+    """One GCN layer (GCN.forward, reference models/other_models.py:61-76): out = LN2(res + drop(act(LN(A_hat x W^T +
+    b)))), where res = x when `residual`; LN / LN2 optional; drop = dropout (p, seed, site) or nothing when dropout is
+    None.  adj_t: the transpose of adj (adj itself when symmetric)."""
 
     @staticmethod
-    def forward(ctx, x, W, bias, ln_w, ln_b, ln2_w, ln2_b, adj, adj_t, relu, residual):
+    def forward(ctx, x, W, bias, ln_w, ln_b, ln2_w, ln2_b, adj, adj_t, relu, residual, dropout=None):
         xw = ops.linear(x, W)
         ln = None if ln_w is None else (ln_w, ln_b)
         ln2 = None if ln2_w is None else (ln2_w, ln2_b)
-        out = ops.gcn_layer(adj, xw, bias, ln=ln, relu=relu, residual=x if residual else None, ln2=ln2)
-        ctx.adj, ctx.adj_t, ctx.relu, ctx.residual = adj, adj_t, relu, residual
+        out = ops.gcn_layer(adj, xw, bias, ln=ln, relu=relu, residual=x if residual else None, ln2=ln2, dropout=dropout)
+        ctx.adj, ctx.adj_t, ctx.relu, ctx.residual, ctx.dropout = adj, adj_t, relu, residual, dropout
         ctx.has_ln, ctx.has_ln2 = ln is not None, ln2 is not None
         ctx.save_for_backward(x, xw, W, bias, ln_w, ln_b, ln2_w, ln2_b)
         return out
@@ -110,15 +119,17 @@ class GCNLayerFunction(torch.autograd.Function):
         g_ln2 = g_ln2b = g_ln = g_lnb = None
         du = dout
         if ctx.has_ln2:
-            if ctx.has_ln or ctx.relu or ctx.residual:
-                u = ops.layernorm_act(y, ln_w, ln_b, relu=ctx.relu, residual=x if ctx.residual else None)
+            if ctx.has_ln or ctx.relu or ctx.residual or ctx.dropout is not None:
+                u = ops.layernorm_act(y, ln_w, ln_b, relu=ctx.relu, residual=x if ctx.residual else None,
+                                      dropout=ctx.dropout)
             else:
                 u = y
             g_ln2, g_ln2b = _zeros_like(ln2_w), _zeros_like(ln2_b)
             du = ops.layernorm_act_backward(u, ln2_w, ln2_b, dout, relu=False, dweight=g_ln2, dbias=g_ln2b)
         if ctx.has_ln:
             g_ln, g_lnb = _zeros_like(ln_w), _zeros_like(ln_b)
-        dy = ops.layernorm_act_backward(y, ln_w, ln_b, du, relu=ctx.relu, dweight=g_ln, dbias=g_lnb)
+        dd = du if ctx.dropout is None else ops.dropout(_rowmajor(du), *ctx.dropout)     # (du may be autograd's dout)
+        dy = ops.layernorm_act_backward(y, ln_w, ln_b, dd, relu=ctx.relu, dweight=g_ln, dbias=g_lnb)
         dxw = ops.gcn_spmm(ctx.adj_t, dy, None)
         dW, db = _zeros_like(W), _zeros_like(bias)
         ops.gemm_wgrad(x, dxw, dW=dW)
@@ -128,7 +139,21 @@ class GCNLayerFunction(torch.autograd.Function):
             dx = ops.linear_dgrad(dxw, W)
             if ctx.residual:
                 ops.layernorm_act_backward(du, None, None, du, relu=False, dx=dx, accumulate_dx=True)   # dx += du
-        return dx, dW, db, g_ln, g_lnb, g_ln2, g_ln2b, None, None, None, None
+        return dx, dW, db, g_ln, g_lnb, g_ln2, g_ln2b, None, None, None, None, None
+
+
+class DropoutFunction(torch.autograd.Function):
+    """x * mask / (1 - p) of (seed, site), row = row of x (the feature dropout in front of the first GCN layer).  The
+    dropped rows are the output (the next layer saves them for its weight gradient); the backward regenerates the mask."""
+
+    @staticmethod
+    def forward(ctx, x, p, seed, site):
+        ctx.drop = (p, seed, site)
+        return ops.dropout(_rowmajor(x), p, seed, site)
+
+    @staticmethod
+    def backward(ctx, dout):
+        return ops.dropout(_rowmajor(dout.float()), *ctx.drop), None, None, None
 
 
 # ------------------------------------------------------------------------------------------------------- link gathers
@@ -211,9 +236,9 @@ class PairwiseFunction(torch.autograd.Function):
     the counts carry no gradient).  Returns [n, H*C + count_dim] (and the per-pair attention weights when asked)."""
 
     @staticmethod
-    def forward(ctx, X, model, batch, sel, idx, want_alpha, *params):
-        feats, alpha, st = model._attention_stack(batch, X, sel, idx, want_alpha=want_alpha, save=True)
-        ctx.model, ctx.sel, ctx.st, ctx.n_params = model, sel, st, len(params)
+    def forward(ctx, X, model, batch, sel, idx, want_alpha, drop, *params):
+        feats, alpha, st = model._attention_stack(batch, X, sel, idx, want_alpha=want_alpha, save=True, drop=drop)
+        ctx.model, ctx.sel, ctx.st, ctx.n_params, ctx.drop = model, sel, st, len(params), drop
         ctx.save_for_backward(X, batch, idx)
         if alpha is not None:
             ctx.mark_non_differentiable(alpha)
@@ -240,9 +265,12 @@ class PairwiseFunction(torch.autograd.Function):
         # the shared (0, 0) rows' gradients, per layer (lpf_attend_backward adds into a contiguous [3, H*C] table)
         dRc = [torch.zeros((3, hc), dtype=torch.float32, device=dev) for hc in HCs] if r_map is not None else None
         g = ops._rowmajor(dfeats.float()[:, : HCs[-1]])
+        drop = ctx.drop
         dxsum = None
         for l in range(L - 1, -1, -1):
             layer = model.att_layers[l]
+            if drop is not None and drop[0][l] > 0:     # layer l's output was dropped: the same mask on its gradient
+                g = ops.dropout(g, drop[0][l], drop[1], ops.SITE_ATT + l, out=None if l == L - 1 else g)
             att = layer.att
             C, HC = att.out_channels, HCs[l]
             Q, R, r_const, feats_in = st["Q"][l], st["R"][l], st["r_const"][l], st["feats_in"][l]
@@ -318,7 +346,7 @@ class PairwiseFunction(torch.autograd.Function):
                     grads[(l, "bias")], grads[(l, "ln_w")], grads[(l, "ln_b")]]
         for g1 in enc_grads:
             out += g1
-        return (dX, None, None, None, None, None, *out)
+        return (dX, None, None, None, None, None, None, *out)
 
 
 def require_training_inputs(*tensors):

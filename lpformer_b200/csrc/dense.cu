@@ -131,12 +131,19 @@ __global__ void __launch_bounds__(256) gemm_simt_kernel(const float* __restrict_
 // ---------------------------------------------------------------------------------------
 // Row-wise LayerNorm (+ReLU, +residual); one warp per row, two-pass statistics.
 // ---------------------------------------------------------------------------------------
+// DROP: dropout after the activation, before the residual (the GCN epilogue of lpf_gcn_layer_dropout); mask row =
+// row0 + r, column = c (rule in common.cuh)
+template <bool DROP>
 __global__ void __launch_bounds__(256) layernorm_act_kernel(const float* X, int64_t ldx,
                                                             const float* __restrict__ g, const float* __restrict__ b,
                                                             const float* R, int64_t ldr,
                                                             float* Y, int64_t ldy, int64_t rows, int n,
-                                                            int relu, const int64_t* __restrict__ rows_dev) {
+                                                            int relu, const int64_t* __restrict__ rows_dev,
+                                                            int64_t row0, const uint64_t* seed_p, int site, uint64_t thr,
+                                                            float scale) {
     if (rows_dev) rows = min(rows, *rows_dev);
+    uint64_t seed = 0;
+    if constexpr (DROP) seed = *seed_p;
     const int lane = threadIdx.x & 31;
     const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
@@ -158,6 +165,7 @@ __global__ void __launch_bounds__(256) layernorm_act_kernel(const float* X, int6
         for (int c = lane; c < n; c += 32) {
             float y = g ? fmaf((x[c] - mean) * rstd, __ldg(g + c), __ldg(b + c)) : x[c];
             if (relu) y = fmaxf(y, 0.f);
+            if constexpr (DROP) y = dropout_apply(y, uint4_word(dropout_bits(seed, site, row0 + r, c >> 2), c & 3), thr, scale);
             if (R) y += R[r * ldr + c];
             Y[r * ldy + c] = y;
         }
@@ -309,9 +317,27 @@ extern "C" int lpf_layernorm_act(const float* X, int64_t ldx, const float* gamma
     LPF_REQUIRE(X && Y, "NULL argument");
     LPF_REQUIRE((gamma == nullptr) == (beta == nullptr), "gamma and beta must both be given or both NULL");
     LPF_REQUIRE(ldx >= n && ldy >= n && (!residual || ldr >= n), "leading dimension too small");
-    layernorm_act_kernel<<<warp_grid(rows, 256), 256, 0, (cudaStream_t)stream>>>(X, ldx, gamma, beta, residual, ldr, Y,
-                                                                                 ldy, rows, n, relu, rows_dev);
+    layernorm_act_kernel<false><<<warp_grid(rows, 256), 256, 0, (cudaStream_t)stream>>>(
+        X, ldx, gamma, beta, residual, ldr, Y, ldy, rows, n, relu, rows_dev, 0, nullptr, 0, 0, 0.f);
     return check_launch("lpf_layernorm_act");
+}
+
+extern "C" int lpf_layernorm_act_dropout(const float* X, int64_t ldx, const float* gamma, const float* beta, int relu,
+                                         int64_t row0, const uint64_t* seed, int32_t site, double p,
+                                         const float* residual, int64_t ldr, float* Y, int64_t ldy, int64_t rows,
+                                         int32_t n, void* stream) {
+    uint64_t thr;
+    float scale;
+    LPF_REQUIRE(dropout_rule(p, &thr, &scale), "p must be in [0, 1]");
+    LPF_REQUIRE(rows >= 0 && n >= 1 && row0 >= 0, "bad shape");
+    LPF_REQUIRE(seed, "seed is NULL");
+    if (rows == 0) return LPF_OK;
+    LPF_REQUIRE(X && Y, "NULL argument");
+    LPF_REQUIRE((gamma == nullptr) == (beta == nullptr), "gamma and beta must both be given or both NULL");
+    LPF_REQUIRE(ldx >= n && ldy >= n && (!residual || ldr >= n), "leading dimension too small");
+    layernorm_act_kernel<true><<<warp_grid(rows, 256), 256, 0, (cudaStream_t)stream>>>(
+        X, ldx, gamma, beta, residual, ldr, Y, ldy, rows, n, relu, nullptr, row0, seed, site, thr, scale);
+    return check_launch("lpf_layernorm_act_dropout");
 }
 
 extern "C" int lpf_gather_links(const int64_t* links, int64_t bs, const int32_t* idx, int64_t n, const float* X,

@@ -35,6 +35,11 @@ struct SpmmParams {
     const float* ln2_b;
     float* Y;
     int64_t ldy;
+    // dropout after the activation (DROP kernels only; rule in common.cuh): mask row = node id, column = channel
+    const uint64_t* seed;
+    int site;
+    uint64_t thr;
+    float scale;
 };
 
 // sum over the LPR lanes of a group (LPR a power of two <= 32, groups aligned)
@@ -45,8 +50,10 @@ __device__ __forceinline__ float group_sum(float v) {
     return v;
 }
 
-// LPR lanes x CH float4 chunks hold one feature row: d <= 4 * LPR * CH, d % 4 == 0 (chunks beyond d are masked)
-template <int LPR, int CH>
+// LPR lanes x CH float4 chunks hold one feature row: d <= 4 * LPR * CH, d % 4 == 0 (chunks beyond d are masked).
+// DROP: dropout between the activation and the residual (GCN.forward: conv -> LN -> dropout -> ReLU -> + residual;
+// dropout and ReLU commute exactly, since relu(m z s) == m relu(z) s for m in {0, 1} and s > 0).
+template <int LPR, int CH, bool DROP>
 __global__ void __launch_bounds__(256, 4) gcn_spmm_kernel(const __grid_constant__ SpmmParams p) {
     constexpr int GW = 32 / LPR;          // neighbour rows per load instruction
     constexpr int UN = 4;                 // load instructions in flight (8 measured: no faster)
@@ -55,6 +62,8 @@ __global__ void __launch_bounds__(256, 4) gcn_spmm_kernel(const __grid_constant_
     const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
     const int d = p.d;
+    uint64_t seed = 0;
+    if constexpr (DROP) seed = *p.seed;
     bool ok[CH];                          // this lane's chunk q lies inside the row
 #pragma unroll
     for (int q = 0; q < CH; ++q) ok[q] = 4 * (gl + q * LPR) < d;
@@ -139,6 +148,17 @@ __global__ void __launch_bounds__(256, 4) gcn_spmm_kernel(const __grid_constant_
 #pragma unroll
                 for (int e = 0; e < 4; ++e) v[q][e] = fmaxf(v[q][e], 0.f);
         }
+        if constexpr (DROP) {
+#pragma unroll
+            for (int q = 0; q < CH; ++q) {
+                if (!ok[q]) continue;
+                const uint4 u = dropout_bits(seed, p.site, row, gl + q * LPR);
+                v[q][0] = dropout_apply(v[q][0], u.x, p.thr, p.scale);
+                v[q][1] = dropout_apply(v[q][1], u.y, p.thr, p.scale);
+                v[q][2] = dropout_apply(v[q][2], u.z, p.thr, p.scale);
+                v[q][3] = dropout_apply(v[q][3], u.w, p.thr, p.scale);
+            }
+        }
         if (p.residual) {
 #pragma unroll
             for (int q = 0; q < CH; ++q) {
@@ -185,6 +205,18 @@ static bool aligned16(const void* q) { return (reinterpret_cast<uintptr_t>(q) & 
 // widths the vectorised kernel takes: multiples of 4 up to 512
 static bool spmm_vec_shape(int d) { return d % 4 == 0 && d >= 4 && d <= 512; }
 
+template <bool DROP>
+static int launch_vec(const SpmmParams& p, unsigned blocks, cudaStream_t st) {
+    if (p.d <= 16) gcn_spmm_kernel<4, 1, DROP><<<blocks, 256, 0, st>>>(p);
+    else if (p.d <= 32) gcn_spmm_kernel<8, 1, DROP><<<blocks, 256, 0, st>>>(p);
+    else if (p.d <= 64) gcn_spmm_kernel<16, 1, DROP><<<blocks, 256, 0, st>>>(p);
+    else if (p.d <= 128) gcn_spmm_kernel<32, 1, DROP><<<blocks, 256, 0, st>>>(p);
+    else if (p.d <= 256) gcn_spmm_kernel<32, 2, DROP><<<blocks, 256, 0, st>>>(p);
+    else if (p.d <= 384) gcn_spmm_kernel<32, 3, DROP><<<blocks, 256, 0, st>>>(p);
+    else gcn_spmm_kernel<32, 4, DROP><<<blocks, 256, 0, st>>>(p);
+    return check_launch("lpf_gcn_spmm");
+}
+
 static int launch_spmm(const SpmmParams& p, bool fused_requested, cudaStream_t st) {
     const bool vec = spmm_vec_shape(p.d) && p.ld_xw % 4 == 0 && p.ldy % 4 == 0 && aligned16(p.XW) && aligned16(p.Y) &&
                      (!p.bias || aligned16(p.bias)) && (!p.residual || (aligned16(p.residual) && p.ld_res % 4 == 0)) &&
@@ -204,14 +236,8 @@ static int launch_spmm(const SpmmParams& p, bool fused_requested, cudaStream_t s
         gcn_spmm_scalar_kernel<<<(unsigned)blocks, 256, 0, st>>>(p);
         return check_launch("lpf_gcn_spmm");
     }
-    if (p.d <= 16) gcn_spmm_kernel<4, 1><<<(unsigned)blocks, 256, 0, st>>>(p);
-    else if (p.d <= 32) gcn_spmm_kernel<8, 1><<<(unsigned)blocks, 256, 0, st>>>(p);
-    else if (p.d <= 64) gcn_spmm_kernel<16, 1><<<(unsigned)blocks, 256, 0, st>>>(p);
-    else if (p.d <= 128) gcn_spmm_kernel<32, 1><<<(unsigned)blocks, 256, 0, st>>>(p);
-    else if (p.d <= 256) gcn_spmm_kernel<32, 2><<<(unsigned)blocks, 256, 0, st>>>(p);
-    else if (p.d <= 384) gcn_spmm_kernel<32, 3><<<(unsigned)blocks, 256, 0, st>>>(p);
-    else gcn_spmm_kernel<32, 4><<<(unsigned)blocks, 256, 0, st>>>(p);
-    return check_launch("lpf_gcn_spmm");
+    if (p.seed) return launch_vec<true>(p, (unsigned)blocks, st);
+    return launch_vec<false>(p, (unsigned)blocks, st);
 }
 
 }  // namespace lpf
@@ -241,4 +267,22 @@ extern "C" int lpf_gcn_layer(const int64_t* rowptr, const int32_t* col, const fl
                 "LayerNorm weight and bias must both be given or both NULL");
     SpmmParams p{rowptr, col, val, row0, rows, XW, ld_xw, bias, d, ln_w, ln_b, relu, residual, ld_res, ln2_w, ln2_b, Y, ldy};
     return launch_spmm(p, true, (cudaStream_t)stream);
+}
+
+extern "C" int lpf_gcn_layer_dropout(const int64_t* rowptr, const int32_t* col, const float* val, int64_t row0,
+                                     int64_t rows, const float* XW, int64_t ld_xw, const float* bias, int32_t d,
+                                     const float* ln_w, const float* ln_b, int relu, const uint64_t* seed, int32_t site,
+                                     double p, const float* residual, int64_t ld_res, const float* ln2_w,
+                                     const float* ln2_b, float* Y, int64_t ldy, void* stream) {
+    LPF_REQUIRE(rows >= 0 && row0 >= 0, "negative row range");
+    SpmmParams prm{rowptr, col, val, row0, rows, XW, ld_xw, bias, d, ln_w, ln_b, relu, residual, ld_res, ln2_w, ln2_b, Y, ldy,
+                   seed, site, 0, 0.f};
+    LPF_REQUIRE(dropout_rule(p, &prm.thr, &prm.scale), "p must be in [0, 1]");
+    LPF_REQUIRE(seed, "seed is NULL");
+    if (rows == 0) return LPF_OK;
+    LPF_REQUIRE(rowptr && XW && Y, "NULL argument");
+    LPF_REQUIRE(d >= 1 && ld_xw >= d && ldy >= d && (!residual || ld_res >= d), "bad d / leading dimension");
+    LPF_REQUIRE((ln_w == nullptr) == (ln_b == nullptr) && (ln2_w == nullptr) == (ln2_b == nullptr),
+                "LayerNorm weight and bias must both be given or both NULL");
+    return launch_spmm(prm, true, (cudaStream_t)stream);
 }

@@ -8,9 +8,10 @@ into src/train's eval loops (train/testing.py:14-121) and loads reference checkp
 behind include/lpformer_b200.h; there is no PyTorch or CPU fallback.
 
 A module in training mode with grad mode enabled builds an autograd graph through the same kernels (autograd.py; the
-backward kernels are in csrc/backward.cu), so the reference's training loop body runs at dropout 0.  In eval mode or
-under torch.no_grad() the outputs are detached, as before.  score_links / score_queries / LinkScoreStream and the plans
-are inference-only.
+backward kernels are in csrc/backward.cu), so the reference's training loop body runs.  In training mode every dropout
+of the reference is applied on the device (csrc/dropout.cu): feat_drop, gnn_drop, the attention layers' dropout,
+MLP / mlp_score dropout and node dropout (att_drop), with or without grad mode.  In eval mode or under torch.no_grad()
+the outputs are detached, as before.  score_links / score_queries / LinkScoreStream and the plans are inference-only.
 """
 from __future__ import annotations
 
@@ -29,11 +30,25 @@ from ._lib import EPI_NONE, EPI_RELU, EPI_SIGMOID, LpfError
 from .graph import CSR, csr_from_sparse, gcn_normalise, transpose_csr
 
 
-def _no_training(module: nn.Module, what: str):
-    if module.training and what:
-        raise NotImplementedError(
-            f"lpformer_b200 is the inference path; {what} (training-time behaviour) is not implemented. "
-            "Call .eval() first.")
+def _drop_p(module: nn.Module, p, *tensors) -> float:
+    """The dropout probability a forward of `module` applies: p in training mode, 0 in eval mode (F.dropout semantics:
+    p outside [0, 1] raises ValueError).  The masks exist on the device only: with p > 0 in training mode a CPU tensor
+    raises NotImplementedError."""
+    ops.check_p(p)
+    if not module.training or p == 0:
+        return 0.0
+    for t in tensors:
+        if t is not None and not t.is_cuda:
+            raise NotImplementedError("dropout runs on the device only (lpformer_b200 has no CPU path); got a "
+                                      f"{t.device} tensor")
+    return float(p)
+
+
+def _seed(module: nn.Module, device):
+    """Draws the module's dropout seed for this forward (kept as module.dropout_seed: the masks of the forward are
+    ops.dropout_mask(module.dropout_seed, site, ...))."""
+    module.dropout_seed = ops.draw_seed(device)
+    return module.dropout_seed
 
 
 def _differentiable(module: nn.Module) -> bool:
@@ -106,12 +121,16 @@ class MLP(nn.Module):
 
     @_grad_if_training
     def forward(self, x, out=None):
-        _no_training(self, "dropout" if self.dropout > 0 else "")
+        p = _drop_p(self, self.dropout, x)
         lead = x.shape[:-1]
         x = x.reshape(-1, x.shape[-1])
-        if torch.is_grad_enabled():
+        if torch.is_grad_enabled() or p > 0:
             AG.require_training_inputs(x)
-            x = AG.MLPFunction.apply(x, self.norm is not None, self.sigmoid, *AG.mlp_params(self.linears, self.norm))
+            seed = _seed(self, x.device) if p > 0 else None
+            x = AG.MLPFunction.apply(x, self.norm is not None, self.sigmoid, p, seed,
+                                     *AG.mlp_params(self.linears, self.norm))
+            if out is not None:
+                out.copy_(x)
             return x.reshape(*lead, x.shape[-1]).squeeze(-1)
         for lin in list(self.linears)[:-1]:
             if self.norm is not None:
@@ -146,11 +165,13 @@ class mlp_score(nn.Module):
 
     @_grad_if_training
     def forward(self, x, return_logits=False):
-        _no_training(self, "dropout" if self.dropout > 0 else "")
+        p = _drop_p(self, self.dropout, x)
         x = x.reshape(-1, x.shape[-1])
-        if torch.is_grad_enabled():
+        if torch.is_grad_enabled() or p > 0:
             AG.require_training_inputs(x)
-            return AG.MLPFunction.apply(x, False, not return_logits, *AG.mlp_params(self.lins, None)).squeeze(-1)
+            seed = _seed(self, x.device) if p > 0 else None
+            return AG.MLPFunction.apply(x, False, not return_logits, p, seed,
+                                        *AG.mlp_params(self.lins, None)).squeeze(-1)
         for lin in list(self.lins)[:-1]:
             x = ops.linear(x, lin.weight, lin.bias, epilogue=EPI_RELU)
         last = self.lins[-1]
@@ -216,8 +237,11 @@ class GCN(nn.Module):
     def forward(self, x, adj_norm: CSR, final_norm=None):
         """reference :61-76.  Per layer one contraction (x W^T) and ONE launch for the rest (SpMM + bias + LayerNorm +
         ReLU + residual, ops.gcn_layer); final_norm = (weight, bias) of a LayerNorm applied to the last layer's output
-        in the same launch (LinkTransformer.gnn_norm)."""
-        _no_training(self, "dropout" if self.dropout > 0 else "")
+        in the same launch (LinkTransformer.gnn_norm).  Dropout (training mode, p = self.dropout) of every layer's
+        activated rows rides in the same launch: mask (seed, SITE_GCN + layer), row = node id."""
+        p = _drop_p(self, self.dropout, x)
+        seed = _seed(self, x.device) if p > 0 else None
+        drop = (lambda i: (p, seed, ops.SITE_GCN + i) if p > 0 else None)   # noqa: E731
         last = len(self.convs) - 1
         if torch.is_grad_enabled():
             AG.require_training_inputs(x)
@@ -228,14 +252,14 @@ class GCN(nn.Module):
                 x = AG.GCNLayerFunction.apply(x, conv.lin.weight, conv.bias, None if ln is None else ln.weight,
                                               None if ln is None else ln.bias, None if ln2 is None else ln2[0],
                                               None if ln2 is None else ln2[1], adj_norm, adj_t, self.relu,
-                                              bool(self.residual and x.shape[-1] == conv.lin.weight.shape[0]))
+                                              bool(self.residual and x.shape[-1] == conv.lin.weight.shape[0]), drop(i))
             return x
         for i, conv in enumerate(self.convs):
             xw = ops.linear(x, conv.lin.weight)
             ln = self.lns[i] if self.lns is not None else None
             res = x if (self.residual and x.shape[-1] == xw.shape[-1]) else None
             x = ops.gcn_layer(adj_norm, xw, conv.bias, ln=None if ln is None else (ln.weight, ln.bias), relu=self.relu,
-                              residual=res, ln2=final_norm if i == last else None)
+                              residual=res, ln2=final_norm if i == last else None, dropout=drop(i))
         return x
 
 
@@ -255,7 +279,16 @@ class NodeEncoder(nn.Module):
 
     @_grad_if_training
     def forward(self, features, adj_norm: CSR, test_set=False, final_norm=None):
-        _no_training(self, "feature dropout" if self.feat_drop > 0 else "")
+        """Feature dropout (training mode, p = feat_drop; mask (seed, SITE_FEATURE), row = node id) in front of the GCN.
+        The dropped features are stored (the first GCN layer saves its input for its weight gradient): one extra
+        [N, F] fp32 table while the graph lives."""
+        p = _drop_p(self, self.feat_drop, features)
+        if p > 0:
+            seed = _seed(self, features.device)
+            if torch.is_grad_enabled():
+                features = AG.DropoutFunction.apply(features, p, seed, ops.SITE_FEATURE)
+            else:
+                features = ops.dropout(ops._rowmajor(features), p, seed, ops.SITE_FEATURE)
         return self.gnn_encoder(features, adj_norm, final_norm=final_norm)
 
 
@@ -542,8 +575,13 @@ class LinkTransformer(nn.Module):
 
     @torch.no_grad()
     def compute_node_mask(self, batch, test_set, adj):
-        """reference :214-276, same return format: per type (ix int64 [2,S_t], src_ppr, tgt_ppr) or None."""
-        sel = self._select(ops.links_tensor(batch, self._dev()), test_set, adj, want_link=True)
+        """reference :214-276, same return format: per type (ix int64 [2,S_t], src_ppr, tgt_ppr) or None.  In training
+        mode with att_drop > 0 the sets are those left by node dropout (reference :257-260).  Its seed is the first draw
+        from the CUDA generator, as in calc_pairwise, so after the same torch.manual_seed both keep the same pairs."""
+        batch = ops.links_tensor(batch, self._dev())
+        p_node = _drop_p(self, self.att_drop, batch)
+        node_drop = (p_node, _seed(self, batch.device)) if p_node > 0 else None
+        sel = self._select(batch, test_set, adj, want_link=True, node_drop=node_drop)
         res = []
         for t in range(3):
             produced = t == 0 or (t == 1 and self.mask != "cn") or (t == 2 and self.mask == "all")
@@ -555,8 +593,13 @@ class LinkTransformer(nn.Module):
             res.append((ix, sel.src_ppr[r0:r1], sel.tgt_ppr[r0:r1]))
         return tuple(res)
 
-    def _select(self, batch, test_set, adj_mask=None, want_link=False):
-        _no_training(self, "node dropout (att_drop)" if self.att_drop > 0 else "")
+    def _select(self, batch, test_set, adj_mask=None, want_link=False, node_drop=None):
+        """The selected pairs of the batch; node_drop = (p, seed): then only the pairs node dropout keeps (reference
+        drop_pairwise :322-337: ceil(S (1 - p)) of them, after the >1-hop set is merged in)."""
+        sel = self._select_all(batch, test_set, adj_mask, want_link)
+        return sel if node_drop is None else ops.drop_pairs(sel, *node_drop)
+
+    def _select_all(self, batch, test_set, adj_mask, want_link):
         stored = self.get_adj(test_set, mask=True)
         th = (self.thresh_cn, self.thresh_1hop, self.thresh_non1hop)
         if adj_mask is None:
@@ -577,17 +620,26 @@ class LinkTransformer(nn.Module):
 
         Links whose three node sets are all empty share one pairwise vector (attention output = LayerNorm(bias),
         counts = 0), so the attention + pairwise_lin stack runs only on the compacted list of non-empty links
-        and the constant row is broadcast to the rest."""
+        and the constant row is broadcast to the rest.
+
+        Training mode: node dropout (att_drop) of the selected pairs, and dropout of each attention layer's output
+        (layer.dropout; mask (seed, SITE_ATT + layer), row = batch position).  One seed per call, drawn first (see
+        compute_node_mask).  With attention dropout every link gets its own masked row, so the stack runs on all links."""
         dev = self._dev()
         batch = ops.links_tensor(batch, dev)
+        p_node = _drop_p(self, self.att_drop, batch, X_node)
+        p_att = tuple(_drop_p(layer, layer.dropout, batch, X_node) for layer in self.att_layers)
+        seed = _seed(self, dev) if p_node > 0 or any(p_att) else None
         X_node = self._check_x(X_node)
         bs = batch.shape[1]
-        sel = self._select(batch, test_set, adj_mask, want_link=return_weights)
+        sel = self._select(batch, test_set, adj_mask, want_link=return_weights,
+                           node_drop=(p_node, seed) if p_node > 0 else None)
+        drop = (p_att, seed) if any(p_att) else None
         nnz = sel.nz.numel()
         if torch.is_grad_enabled():
-            return self._pairwise_differentiable(batch, X_node, sel, return_weights)
-        if return_weights or nnz == bs or bs == 0:
-            pw, alpha = self._pairwise_rows(batch, X_node, sel, None, out=out, want_alpha=return_weights)
+            return self._pairwise_differentiable(batch, X_node, sel, return_weights, drop)
+        if return_weights or nnz == bs or bs == 0 or drop is not None:
+            pw, alpha = self._pairwise_rows(batch, X_node, sel, None, out=out, want_alpha=return_weights, drop=drop)
         else:
             alpha = None
             pw = out if out is not None else torch.empty((bs, self.dim), dtype=torch.float32, device=dev)
@@ -607,20 +659,22 @@ class LinkTransformer(nn.Module):
             X_node = X_node.float().contiguous()
         return X_node
 
-    def _pairwise_differentiable(self, batch, X_node, sel, return_weights):
-        """calc_pairwise with autograd (training mode): the empty-set links share one pairwise row, built through the
-        attention bias -> LayerNorm -> pairwise_lin chain once, whose gradient is the sum over those links."""
+    def _pairwise_differentiable(self, batch, X_node, sel, return_weights, drop=None):
+        """calc_pairwise with autograd (training mode): without attention dropout the empty-set links share one pairwise
+        row, built through the attention bias -> LayerNorm -> pairwise_lin chain once, whose gradient is the sum over
+        those links."""
         bs, nnz = sel.bs, sel.nz.numel()
         params = AG.pairwise_params(self)
         alpha = None
-        if return_weights or nnz == bs or bs == 0:
-            res = AG.PairwiseFunction.apply(X_node, self, batch, sel, None, return_weights, *params)
+        if return_weights or nnz == bs or bs == 0 or drop is not None:
+            res = AG.PairwiseFunction.apply(X_node, self, batch, sel, None, return_weights, drop, *params)
             feats, alpha = res if return_weights else (res, None)
             pw = self.pairwise_lin(feats)
         else:
             rows = None
             if nnz > 0:
-                rows = self.pairwise_lin(AG.PairwiseFunction.apply(X_node, self, batch, sel, sel.nz, False, *params))
+                rows = self.pairwise_lin(AG.PairwiseFunction.apply(X_node, self, batch, sel, sel.nz, False, None,
+                                                                   *params))
             pw = AG.ScatterFillFunction.apply(rows, self._pw_const_differentiable(X_node, params), sel.nz, bs)
         att_weights = torch.stack((sel.link.float(), alpha)) if return_weights else None
         return pw, att_weights
@@ -636,17 +690,21 @@ class LinkTransformer(nn.Module):
         would carry a graph that the first backward frees)."""
         empty = torch.zeros((2, 1), dtype=torch.int64, device=self._dev())
         return self.pairwise_lin(AG.PairwiseFunction.apply(X_node, self, empty, self._empty_selection(), None, False,
-                                                           *params))
+                                                           None, *params))
 
-    def _pairwise_rows(self, batch, X_node, sel, idx, out=None, want_alpha=False):
+    def _pairwise_rows(self, batch, X_node, sel, idx, out=None, want_alpha=False, drop=None):
         """RPE -> attention layers -> counts -> pairwise_lin for the batch positions in idx (all links when None).
         Returns ([n, dim] rows in idx order, per-pair attention weights or None)."""
-        feats, alpha, _ = self._attention_stack(batch, X_node, sel, idx, want_alpha)
+        feats, alpha, _ = self._attention_stack(batch, X_node, sel, idx, want_alpha, drop=drop)
         return self.pairwise_lin(feats, out=out), alpha
 
-    def _attention_stack(self, batch, X_node, sel, idx, want_alpha=False, save=False):
+    def _attention_stack(self, batch, X_node, sel, idx, want_alpha=False, save=False, drop=None):
         """RPE -> attention layers -> counts for the batch positions in idx (all links when None): ([n, H*C +
-        count_dim] rows in idx order, per-pair attention weights or None, and with save=True what the backward reads)."""
+        count_dim] rows in idx order, per-pair attention weights or None, and with save=True what the backward reads).
+        drop = ((p of each layer), seed): each layer's [n, H*C] output is dropped before it feeds the next layer (mask
+        rows are batch positions, so idx must be None)."""
+        if drop is not None and idx is not None:
+            raise ValueError("attention dropout runs over every link of the batch (idx must be None)")
         dev = self._dev()
         d, H = self.dim, self.num_heads
         n = sel.bs if idx is None else idx.numel()
@@ -719,6 +777,8 @@ class LinkTransformer(nn.Module):
             ops.attend(sel, kvs[l], R, Q, att.att, att.bias, layer.post_att_norm.weight, layer.post_att_norm.bias,
                        H, C, write_counts=last, out=feats, alpha_out=alpha if last else None, idx=idx,
                        r_map=r_map, r_const=r_const)
+            if drop is not None and drop[0][l] > 0:       # (not the counts)
+                ops.dropout(feats[:, :HC], drop[0][l], drop[1], ops.SITE_ATT + l, out=feats[:, :HC])
         return feats, alpha, st
 
     def _node_tables(self, X_node, kv):

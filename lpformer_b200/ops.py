@@ -141,8 +141,9 @@ def linear(A, W, bias=None, bias_scale=1.0, out=None, epilogue=EPI_NONE):
     return out
 
 
-def layernorm_act(x, weight, bias, relu=False, residual=None, out=None, n=None):
-    """out = residual + act(LayerNorm(x[:, :n])) row-wise; weight=None skips the norm."""
+def layernorm_act(x, weight, bias, relu=False, residual=None, out=None, n=None, dropout=None, row0=0):
+    """out = residual + act(LayerNorm(x[:, :n])) row-wise; weight=None skips the norm.  dropout = (p, seed, site):
+    out = residual + drop(act(LayerNorm(x))) with mask rows row0 + r (lpf_layernorm_act_dropout)."""
     require_cuda(x, weight, bias, residual, out)
     x = _rowmajor(x)
     rows = x.shape[0]
@@ -151,6 +152,14 @@ def layernorm_act(x, weight, bias, relu=False, residual=None, out=None, n=None):
         out = torch.empty((rows, n), dtype=torch.float32, device=x.device)
     if residual is not None:
         residual = _rowmajor(residual)
+    if dropout is not None:
+        p, seed, site = dropout
+        check_p(p)
+        require_cuda(seed)
+        call("lpf_layernorm_act_dropout", ptr(x), x.stride(0), ptr(weight), ptr(bias), int(relu), int(row0), ptr(seed),
+             int(site), float(p), ptr(residual), residual.stride(0) if residual is not None else 0, ptr(out),
+             out.stride(0), rows, n, stream())
+        return out
     call("lpf_layernorm_act", ptr(x), x.stride(0), ptr(weight), ptr(bias), ptr(residual),
          residual.stride(0) if residual is not None else 0, ptr(out), out.stride(0), rows, n, int(relu), None, stream())
     return out
@@ -507,13 +516,18 @@ def link_heads(links, X, consts, prob, idx=None, zb=None, logits=False, sched=No
     return prob
 
 
-def gcn_layer(adj: CSR, XW, bias, ln=None, relu=False, residual=None, ln2=None, out=None, row0=0, rows=None, local=False):
+def gcn_layer(adj: CSR, XW, bias, ln=None, relu=False, residual=None, ln2=None, out=None, row0=0, rows=None, local=False,
+              dropout=None):
     """One GCN layer after its Linear, in one launch (lpf_gcn_layer): out = LN2(residual + act(LN(A_hat XW + bias)))
     for rows [row0, row0 + rows).  ln / ln2: (weight, bias) or None.  local=False: `out` and `residual` are [n, d]
     tables indexed by node id; local=True: they hold only the rows of the range (row 0 = node row0: the row-sharded
-    multi-GPU layers).  Falls back to lpf_gcn_spmm + lpf_layernorm_act for widths / alignments the fused kernel does
-    not take."""
+    multi-GPU layers).  dropout = (p, seed, site): out = LN2(residual + drop(act(LN(...)))), mask row = node id
+    (lpf_gcn_layer_dropout).  Falls back to lpf_gcn_spmm + lpf_layernorm_act for widths / alignments the fused kernel
+    does not take."""
     require_cuda(adj.rowptr, XW, bias, out, residual)
+    if dropout is not None:
+        check_p(dropout[0])
+        require_cuda(dropout[1])
     XW = _rowmajor(XW)
     n, d = adj.n, XW.shape[1]
     rows = n - row0 if rows is None else rows
@@ -526,6 +540,15 @@ def gcn_layer(adj: CSR, XW, bias, ln=None, relu=False, residual=None, ln2=None, 
     fusable = d % 4 == 0 and d <= 512 and XW.stride(0) % 4 == 0 and out.stride(0) % 4 == 0 and a16(XW) and a16(out) and \
         a16(bias) and (residual is None or (a16(residual) and residual.stride(0) % 4 == 0)) and \
         all(a16(t) for pair in (ln, ln2) if pair is not None for t in pair)
+    if fusable and dropout is not None:
+        call("lpf_gcn_layer_dropout", ptr(adj.rowptr), ptr(adj.col), ptr(adj.val), row0, rows, ptr(XW), XW.stride(0),
+             ptr(bias), d, ptr(ln[0]) if ln else None, ptr(ln[1]) if ln else None, int(relu), ptr(dropout[1]),
+             int(dropout[2]), float(dropout[0]),
+             (residual.data_ptr() - 4 * shift * residual.stride(0)) if residual is not None else None,
+             residual.stride(0) if residual is not None else 0,
+             ptr(ln2[0]) if ln2 else None, ptr(ln2[1]) if ln2 else None,
+             out.data_ptr() - 4 * shift * out.stride(0), out.stride(0), stream(), meta=(rows, d, adj.nnz))
+        return out
     if fusable:
         call("lpf_gcn_layer", ptr(adj.rowptr), ptr(adj.col), ptr(adj.val), row0, rows, ptr(XW), XW.stride(0), ptr(bias), d,
              ptr(ln[0]) if ln else None, ptr(ln[1]) if ln else None, int(relu),
@@ -541,8 +564,9 @@ def gcn_layer(adj: CSR, XW, bias, ln=None, relu=False, residual=None, ln2=None, 
     sh = view[row0:row0 + rows]
     dst = out if local else out[row0:row0 + rows]
     res = None if residual is None else (residual if local else residual[row0:row0 + rows])
-    if ln is not None or relu or res is not None:
-        layernorm_act(sh, None if ln is None else ln[0], None if ln is None else ln[1], relu=relu, residual=res, out=dst)
+    if ln is not None or relu or res is not None or dropout is not None:
+        layernorm_act(sh, None if ln is None else ln[0], None if ln is None else ln[1], relu=relu, residual=res, out=dst,
+                      dropout=dropout, row0=row0)
         sh = dst
     if ln2 is not None:
         layernorm_act(sh, ln2[0], ln2[1], relu=False, out=dst)
@@ -719,3 +743,93 @@ def attend_backward(sel: Selection, KV, R, Q, att, bias, ln_w, ln_b, heads, ch, 
          dR.stride(0) if dR is not None else HC, ptr(dRc), ptr(dQ), HC, ptr(dKV), dKV.stride(0), ptr(rows), stream(),
          meta=(n, sel.total, HC))
     return dQ, rows
+
+
+# ------------------------------------------------------------------------------------------------ dropout (dropout.cu)
+# site numbers of the dropout masks (include/lpformer_b200.h, "Dropout"): a mask is a function of (seed, site, row, col)
+SITE_FEATURE, SITE_NODE, SITE_GCN, SITE_ATT, SITE_MLP = 1, 2, 16, 32, 48
+
+
+def check_p(p):
+    """F.dropout's argument check."""
+    if not 0.0 <= float(p) <= 1.0:
+        raise ValueError(f"dropout probability has to be between 0 and 1, but got {p}")
+
+
+def draw_seed(device):
+    """One 64-bit dropout seed from torch's CUDA generator of `device`, as an int64 [1] device tensor (no host sync):
+    after torch.manual_seed(s) the same sequence of seeds, hence of masks, comes back."""
+    return torch.randint(-2 ** 63, 2 ** 63 - 1, (1,), dtype=torch.int64, device=device)
+
+
+def _seed_tensor(seed, device):
+    if torch.is_tensor(seed):
+        if seed.dtype != torch.int64 or seed.numel() < 1:
+            raise ValueError("seed must be an int64 device tensor")
+        require_cuda(seed)
+        return seed
+    return torch.tensor([int(seed) - (1 << 64) if int(seed) >= 1 << 63 else int(seed)], dtype=torch.int64, device=device)
+
+
+def dropout(x, p, seed, site, row0=0, out=None):
+    """out = x * mask / (1 - p) (lpf_dropout) over the rows of a 2-D fp32 tensor with unit column stride (any row stride);
+    mask row = row0 + r.  out=x: in place.  seed: an int64 device tensor (draw_seed) or a Python int."""
+    check_p(p)
+    require_cuda(x, out)
+    if x.dtype != torch.float32 or x.dim() != 2 or (x.shape[1] > 1 and x.stride(1) != 1):
+        raise ValueError("dropout: x must be a 2-D fp32 tensor with unit column stride")
+    rows, n = x.shape
+    if out is None:
+        out = torch.empty((rows, n), dtype=torch.float32, device=x.device)
+    elif out.shape != x.shape or out.dtype != torch.float32 or (n > 1 and out.stride(1) != 1):
+        raise ValueError("dropout: bad `out`")
+    if rows == 0 or n == 0:
+        return out
+    seed = _seed_tensor(seed, x.device)
+    call("lpf_dropout", ptr(x), max(x.stride(0), n), ptr(out), max(out.stride(0), n), rows, n, int(row0), ptr(seed),
+         int(site), float(p), stream(), meta=(rows, n))
+    return out
+
+
+def dropout_mask(seed, site, rows, n, p, row0=0, device="cuda"):
+    """The [rows, n] mask of (seed, site) for rows row0 .. row0 + rows, times 1 / (1 - p): lpf_dropout applied to ones
+    (the inspection hook of the tests)."""
+    dev = seed.device if torch.is_tensor(seed) else torch.device(device)
+    return dropout(torch.ones((rows, n), dtype=torch.float32, device=dev), p, seed, site, row0=row0)
+
+
+def drop_pairs(sel: Selection, p, seed, site=SITE_NODE) -> Selection:
+    """Node dropout of a selection (reference drop_pairwise): keeps exactly K = ceil(S (1 - p)) of its S pairs, a uniform
+    K-subset drawn from (seed, site), in their order (lpf_drop_pairs_count / _fill), and rebuilds ptr, bounds and nz.
+    One host read (the new bounds and the count of non-empty links)."""
+    import math
+    check_p(p)
+    S, bs = sel.total, sel.bs
+    K = math.ceil(S * (1.0 - float(p)))
+    if K == S:
+        return sel
+    dev = sel.ptr.device
+    seed = _seed_tensor(seed, dev)
+    require_cuda(sel.ptr, sel.node, seed)
+    ws = torch.empty(_lib.load().lpf_drop_pairs_workspace_bytes() // 8 + 1, dtype=torch.int64, device=dev)
+    counts = torch.empty(3 * bs, dtype=torch.int32, device=dev)
+    st = stream()
+    call("lpf_drop_pairs_count", ptr(sel.ptr), bs, S, K, ptr(seed), int(site), ptr(counts), ptr(ws), 8 * ws.numel(), st,
+         meta=(bs, S), launches=18 if K > 0 else 2)
+    p_out = torch.empty(3 * bs + 1, dtype=torch.int64, device=dev)
+    scratch = torch.empty(max(1, _lib.load().lpf_scan_scratch_bytes(3 * bs) // 8), dtype=torch.int64, device=dev)
+    call("lpf_scan_counts", ptr(counts), 3 * bs, ptr(p_out), ptr(scratch), st)
+    nz = torch.empty(bs, dtype=torch.int32, device=dev)
+    header = torch.empty(4, dtype=torch.int64, device=dev)
+    call("lpf_select_compact", ptr(p_out), bs, ptr(nz), ptr(header), st)
+    b = header.tolist()          # (S_cn, S_cn + S_1hop, K, #non-empty links)
+    if b[2] != K:
+        raise _lib.LpfError(f"node dropout kept {b[2]} pairs instead of {K}")
+    node = torch.empty(K, dtype=torch.int32, device=dev)
+    pa = torch.empty(K, dtype=torch.float32, device=dev)
+    pb = torch.empty(K, dtype=torch.float32, device=dev)
+    link = torch.empty(K, dtype=torch.int32, device=dev) if sel.link is not None else None
+    if K > 0:
+        call("lpf_drop_pairs_fill", ptr(sel.ptr), bs, ptr(sel.node), ptr(sel.src_ppr), ptr(sel.tgt_ppr), ptr(sel.link),
+             S, ptr(seed), int(site), ptr(ws), ptr(p_out), ptr(node), ptr(pa), ptr(pb), ptr(link), st, meta=(bs, K))
+    return Selection(sel.mode, bs, p_out, node, pa, pb, link, (0, b[0], b[1], b[2]), nz[:b[3]])

@@ -11,7 +11,11 @@ split (CUDA events around every C-ABI call of one further traced step, summed pe
 among the timed ones), peak device memory of a step, and the GPU's name, power limit and max SM clock (read-only
 nvidia-smi query in the same run).
 
-  python tools/train_step_bench.py [--links 32768 --steps 5 --warmup 2]
+With --feat-drop / --gnn-drop / --dropout / --att-drop / --pred-dropout (all 0 by default) the modules train with
+those dropouts (the reference's run-script arguments of the same names; --pred-dropout is mlp_score's), and the line
+gains a "dropout" field.
+
+  python tools/train_step_bench.py [--links 32768 --steps 5 --warmup 2] [--feat-drop 0.1 --gnn-drop 0.1 ...]
 """
 from __future__ import annotations
 
@@ -38,6 +42,8 @@ def parse():
     ap.add_argument("--warmup", type=int, default=2)
     ap.add_argument("--scale", type=float, default=1.0)
     ap.add_argument("--seed", type=int, default=0)
+    for name in ("feat-drop", "gnn-drop", "dropout", "att-drop", "pred-dropout"):
+        ap.add_argument("--" + name, type=float, default=0.0)
     args = ap.parse_args()
     args.workload, args.negs = "citation2", None
     if args.steps < 1 or args.warmup < 1 or args.links < 1:
@@ -66,8 +72,9 @@ def main():
 
     g, negs, _ = B.make_workload(args, 0)
     torch.manual_seed(args.seed)
-    model = L_.LinkTransformer(S.train_args_of(g.cfg), g.data_dict(dev), device=dev).to(dev).train()
-    score = L_.mlp_score(model.out_dim, model.out_dim, 1, 2).to(dev).train()
+    drops = {"feat_drop": args.feat_drop, "gnn_drop": args.gnn_drop, "dropout": args.dropout, "att_drop": args.att_drop}
+    model = L_.LinkTransformer(dict(S.train_args_of(g.cfg), **drops), g.data_dict(dev), device=dev).to(dev).train()
+    score = L_.mlp_score(model.out_dim, model.out_dim, 1, 2, dropout=args.pred_dropout).to(dev).train()
     opt = torch.optim.Adam(list(model.parameters()) + list(score.parameters()), lr=1e-3)
     rng = np.random.default_rng(args.seed)
     E = g.edges.shape[1]
@@ -124,6 +131,8 @@ def main():
         "peak_device_memory_gb": peak / 1e9, "resident_before_step_gb": base / 1e9,
         "losses": losses,
     }
+    if any(drops.values()) or args.pred_dropout:
+        line["dropout"] = dict(drops, pred_dropout=args.pred_dropout)
     print(json.dumps(line))
 
 
